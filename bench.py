@@ -168,6 +168,26 @@ def ncu_traffic():
     return d, os.path.relpath(files[-1], ROOT)
 
 
+# --dump-outputs: at most 56 MB in all, so that two builds can be compared file by file
+DUMP_CAP_BYTES = {"sr": 40_000_000, "l1_features": 16_000_000}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy in float32.  A tensor larger than its DUMP_CAP_BYTES entry is written
+    as a 1-D sample instead: the elements at the sorted flat indices numpy.random.default_rng(0) draws without replacement, which
+    depend only on the tensor's size and so are the same in every run with the same arguments."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.float()
+        cap = DUMP_CAP_BYTES[name] // 4
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------ our arm
 def run_ours(args):
     import torch
@@ -328,6 +348,11 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     ms, l1, launches, dcn_log = timed(step_resident, args.steps, args.warmup, l1, True)
+    if args.dump_outputs and rank == 0:
+        # what forward() returned in the last timed step, before the runs below overwrite the graph's static outputs; the feature
+        # ring hands out its window frame-major, the cat path batch-major: written batch-major [seqs, 7, 64, H, W] either way
+        feats = l1.reshape(7, S, *l1.shape[1:]).transpose(0, 1) if getattr(l1, "_cdfo_ring", None) else l1.reshape(S, 7, *l1.shape[1:])
+        dump_outputs(args.dump_outputs, {"sr": last_sr[0], "l1_features": feats})
     if graphed is not None:
         # inside a replayed graph neither the ctypes launch counter nor the per-launch events exist: take both from eager steps
         keep, graphed = graphed, None
@@ -498,10 +523,17 @@ def run_c4(args):
         dist.destroy_process_group()
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % v)
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--seqs", type=int, default=4, help="independent sequences resident per GPU (batched per step).  8 measured 89.2 / 85.5 HR fps on one GPU and 677 on eight against 85.6 and 699 with 4: about +4 %% per SM clock, less than the spread between power-capped boxes")
@@ -519,7 +551,12 @@ def main():
     ap.add_argument("--cpu-baseline-budget-s", type=int, default=80, help="cap of the in-arm cpu_baseline leg (full frames, rank 0, N = 1)")
     ap.add_argument("--graph", type=int, default=0, help="1: replay the steady-state step as a CUDA graph (+1.7 %%); 0 (default): eager "
                     "launches, which is what lets the DCN kernel be timed live with CUDA events inside the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="c3: after the timed steps, write what the last one returned as DIR/sr.npy (the HR "
+                    "frames [seqs, 1, 4H, 4W]) and DIR/l1_features.npy (the window's L1 features [seqs, 7, 64, H, W]), float32; an output "
+                    "over its size cap is written as a fixed seeded 1-D sample (bench.dump_outputs).  Rank 0's sequences only")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "c4"):
+        ap.error("--dump-outputs writes the outputs of the c3 steps of our arm only")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "c4":

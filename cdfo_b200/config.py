@@ -47,6 +47,9 @@ mdta_c8 = os.environ.get("CDFO_MDTA_C8", "1") != "0"
 # True: the down / up 1x1 convolutions of a cross-scale block are composed into body.0's 3x3 weights (they commute with the bilinear
 # resampling; the 1x1 bias becomes a border-class bias table of the 3x3 kernel's epilogue): 42 fewer launches per trunk.
 trunk_compose_1x1 = os.environ.get("CDFO_TRUNK_COMPOSE_1X1", "1") != "0"
+# With trunk_compose_1x1 and conv_fold_half: True = body.0 of the down(body(up(x))) branch builds its A operand from the 1x image (bilinear x2 in
+# the producer, cdfo_conv3x3_pair_sm100_up2_fwd; bit-identical): the 2x input tensor is never written.  False = resample kernel + convolution.
+trunk_fused_upsample = os.environ.get("CDFO_TRUNK_FUSED_UPSAMPLE", "1") != "0"
 # True: the mask logits of LLongRangAttention start from the ONE-channel residual map (conv_expand_rms composed with conv_du_re.0 + ReLU as one
 # direct 1 -> 64 convolution) instead of reading the 64-channel prior features through a 1x1 convolution kernel.
 lra_logits_from_prior = os.environ.get("CDFO_LRA_LOGITS_FROM_PRIOR", "1") != "0"

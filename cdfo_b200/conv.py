@@ -200,6 +200,28 @@ def conv3x3(x8, weight, bias=None, act=ACT_NONE, resid8=None, out_nchw=False, pi
 
 
 @torch.no_grad()
+def conv3x3_up2(x8, weight, bias, act=ACT_NONE, parity_planes=False, bias_edge=None):
+    """conv3x3(resample(x8, 1), weight, bias, act, parity_planes=..., bias_edge=...) bit for bit, with the bilinear x2 evaluated while the
+    convolution's A operand is built: x8 [B, 8, H, W, 8] bf16 (the 1x image), weight [256, 64, 3, 3] -> [B, 32, 2H, 2W, 8] bf16 (or its
+    parity planes [B, 32, 2, 2, H, W, 8]); bias_edge [9, 256] fp32 as in conv3x3."""
+    B, C8, H, W, _ = x8.shape
+    Cout, Cin = weight.shape[:2]
+    if C8 * 8 != Cin or (Cout, Cin) != (256, 64) or tuple(weight.shape[2:]) != (3, 3):
+        raise _lib.CdfoError("conv3x3_up2: 64 -> 256 3x3 only, got weight %s on input %s" % (tuple(weight.shape), tuple(x8.shape)))
+    if x8.dtype != torch.bfloat16 or not x8.is_contiguous():
+        raise _lib.CdfoError("conv3x3_up2: input must be a contiguous bf16 c8 tensor")
+    b = None if bias is None else bias.detach().contiguous().float()
+    if bias_edge is not None and (b is None or tuple(bias_edge.shape) != (9, Cout) or bias_edge.dtype != torch.float32
+                                  or not bias_edge.is_contiguous()):
+        raise _lib.CdfoError("conv3x3_up2: bias_edge needs a bias and a contiguous fp32 [9, %d] table" % Cout)
+    shape = (B, Cout // 8, 2, 2, H, W, 8) if parity_planes else (B, Cout // 8, 2 * H, 2 * W, 8)
+    y = torch.empty(shape, dtype=torch.bfloat16, device=x8.device)
+    _lib.call("cdfo_conv3x3_pair_sm100_up2_fwd", _lib.ptr(x8), _lib.ptr(pack_weight_pair(weight)), _lib.ptr(b), _lib.ptr(bias_edge), _lib.ptr(y),
+              B, Cin, Cout, 2 * H, 2 * W, int(act), 1 if parity_planes else 0, _lib.stream_ptr(x8.device))
+    return y
+
+
+@torch.no_grad()
 def conv_last_skip(x8, weight, bias, lr):
     """conv_last (Cin -> 1, 3x3) + bias + bilinear x4 skip of the 1-channel LR image lr [B,1,H/4,W/4] (arch:4477-4480).
     x8 [B, Cin/8, H, W, 8] bf16 -> [B, 1, H, W] fp32."""

@@ -14,12 +14,19 @@
 // weights [half][tap][Cin/8][32][8] bf16.  Pipeline: warp 0 = TMA producer (both CTAs; completion bytes of both land on the LEADER's
 // full barrier), warp 1 of the leader = MMA issuer (commits are multicast to both CTAs' barriers), warps 2..9 = epilogue of the
 // CTA's own 128 pixels (bias -> act -> +residual -> c8 bf16), accumulator double-buffered in TMEM (2 x 64 columns per CTA).
+//
+// UP2 (64 -> 256 only, body.0 of Block_'s down(body(up(x))) branch): the input is the 1x image and the A stage is BUILT instead of
+// loaded -- the 18 x 10 halo of bilinear_x2(x) -- by four builder warps (warps 10..13) from a 10 x 6 x 64-channel raw tile of the 1x
+// image in shared memory (7.7 KB instead of 23 KB of L2 -> SM traffic, and no 2x tensor written to and read back from HBM).  The
+// values are those of resample.cu's upsample2_c8_kernel bit for bit (same helpers, up2_blend.cuh), so the convolution's result is too.
 #include <cuda.h>
 #include <stdlib.h>
+#include <string.h>
 
 #include "cdfo_common.cuh"
 #include "sm100_pair.cuh"
 #include "sm100_ptx.cuh"
+#include "up2_blend.cuh"
 
 namespace cdfo {
 namespace cpair {
@@ -30,7 +37,11 @@ constexpr int kSbo = kHaloW * 16;
 constexpr int kChunks = 8;                        // 64 channels per pipeline stage
 constexpr int kABytes = kChunks * kPlane;         // 23 040
 constexpr int kStages = 3;
-constexpr int kThreads = 320, kEpiWarps = 8;
+constexpr int kEpiWarps = 8;
+// UP2: the 1x source of one A stage = source rows h0/2 - 1 .. h0/2 + 8 and columns w0/2 - 1 .. w0/2 + 4 (edge-clamped) of 8 chunks
+constexpr int kRawH = kTileH / 2 + 2, kRawW = kTileW / 2 + 2, kRawPix = kChunks * kRawH * kRawW, kRawBytes = kRawPix * 16;   // 7 680
+constexpr int kBuildWarps = 4, kBuildThreads = kBuildWarps * 32;
+constexpr int threads_of(bool up2) { return (2 + kEpiWarps + (up2 ? kBuildWarps : 0)) * 32; }   // 320 / 448
 
 struct Params {
   const uint8_t *wpk;   // [2 halves][9 taps][Cin/8][NH][8] bf16
@@ -38,6 +49,7 @@ struct Params {
   const float *bias_edge;  // [9][2 NH] or nullptr: the bias of border pixels by class (row top / middle / bottom) * 3 + (column left / middle /
                            // right) -- a 1x1 convolution composed INTO this 3x3 one has its own bias under the taps inside the frame only
   const uint4 *resid;   // c8 bf16 [B][2 NH / 8][H][W][8] or nullptr (added after the activation)
+  const uint4 *x1;      // UP2: the 1x input c8 bf16 [B][8][H/2][W/2][8]; H, W below are the 2x (output) size
   uint4 *y;             // c8 bf16 [B][2 NH / 8][H][W][8]
   int B, Cin, H, W, act;
   int tiles_x, tiles_y, m_tiles;
@@ -48,10 +60,12 @@ struct Params {
 
 using namespace pairptx;
 
-// NH = output channels whose weights one CTA holds (N = 2 NH over the pair)
-template <int NH>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
+// NH = output channels whose weights one CTA holds (N = 2 NH over the pair); UP2: A built from the 1x image (NH = 128, Cin = 64)
+template <int NH, bool UP2>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(threads_of(UP2), 1)
 conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params p) {
+  static_assert(!UP2 || NH == 128, "UP2 is instantiated for 64 -> 256 only");
+  constexpr int kThreads = threads_of(UP2);
   constexpr int kNH = NH, kN = 2 * NH;
   constexpr int kPiece = kNH * 64 * 2;              // weights of one (tap, K block) and CTA
   constexpr int kAccCols = kN, kTmemCols = 2 * kN;  // accumulator double-buffered: 128 or 512 columns
@@ -60,10 +74,11 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
   const int w_bytes = 9 * p.Cin * kNH * 2;                // this CTA's half of the weights
   uint8_t *wsm = smem;
   uint8_t *asmem = smem + ((w_bytes + 1023) & ~1023);
-  uint64_t *bars = reinterpret_cast<uint64_t *>(asmem + kStages * kABytes);
+  uint4 *raw = reinterpret_cast<uint4 *>(asmem + kStages * kABytes);         // UP2 only
+  uint64_t *bars = reinterpret_cast<uint64_t *>(asmem + kStages * kABytes + (UP2 ? kRawBytes : 0));
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 16);
   float *bias_s = reinterpret_cast<float *>(bars + 18);
-  // barrier map: [0,3) A full (leader's is used), [4,7) A empty, 8/9 accumulator full, 10/11 accumulator empty (leader's), 12 weights
+  // barrier map: [0,3) A full (leader's is used; UP2: one arrival per builder warp of both CTAs), [4,7) A empty, 8/9 accumulator full, 10/11 accumulator empty (leader's), 12 weights
   const uint32_t bar0 = ptx::smem_u32(bars);
   auto BAR = [&](int i) { return bar0 + 8u * i; };
 
@@ -75,7 +90,7 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
   for (int i = tid; i < kN; i += kThreads) bias_s[i] = p.bias ? p.bias[i] : 0.f;
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < kStages; ++s) {
-      ptx::mbar_init(BAR(s), 1);
+      ptx::mbar_init(BAR(s), UP2 ? 2 * kBuildWarps : 1);
       ptx::mbar_init(BAR(4 + s), 1);
     }
     for (int a = 0; a < 2; ++a) {
@@ -84,7 +99,7 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
     }
     ptx::mbar_init(BAR(12), 1);
     ptx::fence_mbar_init();
-    ptx::prefetch_tmap(&tmap);
+    if (!UP2) ptx::prefetch_tmap(&tmap);
     ptx::mbar_arrive_expect_tx(BAR(12), w_bytes);
     const uint8_t *src = p.wpk + (size_t)rank * w_bytes;
     for (int i = 0; i < 9 * KB; ++i) ptx::bulk_g2s(ptx::smem_u32(wsm) + i * kPiece, src + (size_t)i * kPiece, kPiece, BAR(12));
@@ -103,7 +118,7 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
 
   if (warp == 0) {
     // =========================== TMA producer (both CTAs, own tile) ===========================
-    if (lane == 0) {
+    if (!UP2 && lane == 0) {
       int stage = 0, phase = 0;
       for (int it = 0;; ++it) {
         const int t0 = (it * num_pairs + pair) * 2;
@@ -176,7 +191,7 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
         if (acc == 0) acc_phase ^= 1;
       }
     }
-  } else {
+  } else if (warp < 2 + kEpiWarps) {
     // =========================== epilogue (both CTAs, own 128 pixels x 64 channels) ===========================
     const int quarter = warp & 3;
     const int ehalf = (warp - 2) >> 2;
@@ -259,6 +274,94 @@ conv3x3_pair_sm100_kernel(const __grid_constant__ CUtensorMap tmap, const Params
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1;
     }
+  } else if (UP2) {
+    // =========================== A builders (UP2: both CTAs, own tile) ===========================
+    const int bt = tid - (2 + kEpiWarps) * 32;
+    const int Hi = p.H >> 1, Wi = p.W >> 1;
+    constexpr int kFetch = (kRawPix + kBuildThreads - 1) / kBuildThreads;     // 4 raw blocks per thread
+    // the stage's 8 chunks x 10 halo columns, 20 per builder warp (one warp per SM sub-partition, the same issue load on each)
+    constexpr int kColsPerWarp = kChunks * kHaloW / kBuildWarps;
+    const bool col_live = lane < kColsPerWarp;
+    const int bcol = (bt >> 5) * kColsPerWarp + lane, bc = bcol / kHaloW, bj = bcol % kHaloW;
+    // the tile of iteration `it`; a pair's odd tile past the end builds tile 0, which is never stored (as the TMA producer loads it)
+    auto tile_of = [&](int it, int &b, int &h0, int &w0) {
+      const int t0 = (it * num_pairs + pair) * 2;
+      if (t0 >= p.m_tiles) return false;
+      const int mt = t0 + (int)rank;
+      b = h0 = w0 = 0;
+      if (mt < p.m_tiles) {
+        b = mt / tiles_per_img;
+        const int r = mt - b * tiles_per_img;
+        h0 = (r / p.tiles_x) * kTileH;
+        w0 = (r % p.tiles_x) * kTileW;
+      }
+      return true;
+    };
+    // raw block (chunk, row, column) of the 10 x 6 source window holds the EDGE-CLAMPED source pixel: bilinear x2 repeats the edge pixel
+    auto fetch = [&](int b, int h0, int w0, uint4 (&v)[kFetch]) {
+#pragma unroll
+      for (int k = 0; k < kFetch; ++k) {
+        const int q = bt + k * kBuildThreads;
+        if (q < kRawPix) {
+          const int c = q / (kRawH * kRawW), rr = (q / kRawW) % kRawH, cc = q % kRawW;
+          const int si = min(max((h0 >> 1) - 1 + rr, 0), Hi - 1), sj = min(max((w0 >> 1) - 1 + cc, 0), Wi - 1);
+          v[k] = __ldg(p.x1 + (((size_t)b * kChunks + c) * Hi + si) * Wi + sj);
+        }
+      }
+    };
+    int b = 0, h0 = 0, w0 = 0, stage = 0, phase = 0;
+    uint4 v[kFetch];
+    bool more = tile_of(0, b, h0, w0);
+    if (more) fetch(b, h0, w0, v);
+    for (int it = 0; more; ++it) {
+#pragma unroll
+      for (int k = 0; k < kFetch; ++k)
+        if (bt + k * kBuildThreads < kRawPix) raw[bt + k * kBuildThreads] = v[k];
+      asm volatile("bar.sync 1, %0;" ::"n"(kBuildThreads) : "memory");      // the raw tile is complete
+      int nb = 0, nh0 = 0, nw0 = 0;
+      more = tile_of(it + 1, nb, nh0, nw0);
+      if (more) fetch(nb, nh0, nw0, v);                   // the next tile's loads are in flight while this one is built
+      ptx::mbar_wait(BAR(4 + stage), phase ^ 1);
+      if (col_live) {
+        // one (chunk, halo column) per lane, walked down the raw rows: each column blend feeds the two 2x rows around its source row
+        uint4 *d = reinterpret_cast<uint4 *>(asmem + stage * kABytes) + bc * (kHaloH * kHaloW) + bj;   // the TMA box's canonical layout
+        const int C = w0 - 1 + bj;                        // 2x column
+        const uint4 zero = make_uint4(0u, 0u, 0u, 0u);    // the convolution's zero padding outside the 2x frame
+        if (C < 0 || C >= p.W) {
+#pragma unroll
+          for (int i = 0; i < kHaloH; ++i) d[i * kHaloW] = zero;
+        } else {
+          // source column C/2 and its neighbour towards the output, as raw-tile indices (the clamped copies do the edge clamp)
+          const int c0 = (C >> 1) - (w0 >> 1) + 1, cn = c0 + ((C & 1) ? 1 : -1);
+          const uint4 *rp = raw + bc * (kRawH * kRawW);
+          up2::F8 prev = up2::blend(up2::unpack(rp[cn]), up2::unpack(rp[c0]));                                    // columns first
+#pragma unroll
+          for (int rr = 1; rr < kRawH; ++rr) {
+            const up2::F8 cur = up2::blend(up2::unpack(rp[rr * kRawW + cn]), up2::unpack(rp[rr * kRawW + c0]));
+            // halo row 2 rr - 2 = odd 2x row R (source row rr - 1, neighbour rr), halo row 2 rr - 1 = even row R + 1 (source rr,
+            // neighbour rr - 1); then rows
+            const int R = h0 + 2 * rr - 3;
+            d[(2 * rr - 2) * kHaloW] = R >= 0 && R < p.H ? up2::pack(up2::blend(cur, prev)) : zero;
+            d[(2 * rr - 1) * kHaloW] = R + 1 < p.H ? up2::pack(up2::blend(prev, cur)) : zero;
+            prev = cur;
+          }
+        }
+      }
+      ptx::fence_proxy_async_smem();                      // generic-proxy stores -> visible to the tensor cores (async proxy)
+      __syncwarp();
+      if (lane == 0) {
+        if (leader) ptx::mbar_arrive(BAR(stage));
+        else mbar_arrive_cluster(BAR(stage), 0);
+      }
+      asm volatile("bar.sync 1, %0;" ::"n"(kBuildThreads) : "memory");      // every builder is done reading the raw tile
+      if (++stage == kStages) { stage = 0; phase ^= 1; }
+      b = nb; h0 = nh0; w0 = nw0;
+    }
+    // the producer's tail: the multicast commits that release the last stages must land before the CTA retires
+    for (int s = 0; s < kStages; ++s) {
+      ptx::mbar_wait(BAR(4 + stage), phase ^ 1);
+      if (++stage == kStages) { stage = 0; phase ^= 1; }
+    }
   }
 
   ptx::tc_fence_before();
@@ -287,14 +390,17 @@ static int half_channels(int Cout, int Cin) {
   if (Cout == 256 && Cin == 64) return 128;
   return 0;
 }
-static size_t smem_bytes(int Cin, int NH) { return (size_t)((9 * Cin * NH * 2 + 1023) & ~1023) + kStages * kABytes + 18 * 8 + 2 * NH * 4 + 64; }
+static size_t smem_bytes(int Cin, int NH, bool up2 = false) {
+  return (size_t)((9 * Cin * NH * 2 + 1023) & ~1023) + kStages * kABytes + (up2 ? kRawBytes : 0) + 18 * 8 + 2 * NH * 4 + 64;
+}
 
-template <int NH>
+template <int NH, bool UP2>
 static int launch(const CUtensorMap &tm, const Params &p, cudaStream_t stream) {
-  const size_t smem = smem_bytes(p.Cin, NH);
+  constexpr int kThreads = threads_of(UP2);
+  const size_t smem = smem_bytes(p.Cin, NH, UP2);
   static size_t attr_smem = 0;
   static int max_pairs = 0;
-  auto kern = conv3x3_pair_sm100_kernel<NH>;
+  auto kern = conv3x3_pair_sm100_kernel<NH, UP2>;
   if (smem > attr_smem) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cudaFuncSetAttribute(conv3x3_pair_sm100<%d>, %zu): %s", NH, smem, cudaGetErrorString(e));
@@ -313,7 +419,7 @@ static int launch(const CUtensorMap &tm, const Params &p, cudaStream_t stream) {
   int pairs = (p.m_tiles + 1) / 2;
   if (pairs > max_pairs) pairs = max_pairs;
   kern<<<pairs * 2, kThreads, smem, stream>>>(tm, p);
-  return check_launch("cdfo_conv3x3_pair_sm100_fwd");
+  return check_launch(UP2 ? "cdfo_conv3x3_pair_sm100_up2_fwd" : "cdfo_conv3x3_pair_sm100_fwd");
 }
 
 }  // namespace cpair
@@ -380,12 +486,36 @@ extern "C" int cdfo_conv3x3_pair_sm100_edge_fwd(const void *x_c8, const void *wp
                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   CDFO_REQUIRE(cr == CUDA_SUCCESS, CDFO_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)cr);
   cpair::Params p;
-  p.wpk = (const uint8_t *)wpk; p.bias = bias; p.bias_edge = bias_edge; p.resid = (const uint4 *)resid_c8; p.y = (uint4 *)y_c8;
+  p.wpk = (const uint8_t *)wpk; p.bias = bias; p.bias_edge = bias_edge; p.resid = (const uint4 *)resid_c8; p.x1 = nullptr; p.y = (uint4 *)y_c8;
   p.B = B; p.Cin = Cin; p.H = H; p.W = W; p.act = act; p.y_planes = y_planes; p.tma_wide = wide ? 1 : 0;
   p.tiles_x = ceil_div(W, cpair::kTileW); p.tiles_y = ceil_div(H, cpair::kTileH);
   const long long mt = (long long)B * p.tiles_x * p.tiles_y;
   CDFO_REQUIRE(mt < (1ll << 30), CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_fwd: too many tiles");
   p.m_tiles = (int)mt;
-  if (cpair::half_channels(Cout, Cin) == 32) return cpair::launch<32>(tm, p, (cudaStream_t)stream);
-  return cpair::launch<128>(tm, p, (cudaStream_t)stream);
+  if (cpair::half_channels(Cout, Cin) == 32) return cpair::launch<32, false>(tm, p, (cudaStream_t)stream);
+  return cpair::launch<128, false>(tm, p, (cudaStream_t)stream);
+}
+
+extern "C" int cdfo_conv3x3_pair_sm100_up2_fwd(const void *x8_1x, const void *wpk, const float *bias, const float *bias_edge, void *y,
+                                               int B, int Cin, int Cout, int H2, int W2, int act, int y_planes, void *stream) {
+  CDFO_REQUIRE(x8_1x && wpk && y, CDFO_ERR_NULL, "cdfo_conv3x3_pair_sm100_up2_fwd: NULL pointer");
+  CDFO_REQUIRE(Cin == 64 && Cout == 256, CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_up2_fwd: unsupported channels %d -> %d (64 -> 256 only)",
+               Cin, Cout);
+  CDFO_REQUIRE(B > 0 && H2 > 0 && W2 > 0 && H2 % 2 == 0 && W2 % 2 == 0, CDFO_ERR_SHAPE,
+               "cdfo_conv3x3_pair_sm100_up2_fwd: the 2x size must be positive and even (got %d x %d)", H2, W2);
+  CDFO_REQUIRE(y_planes == 0 || y_planes == 1, CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_up2_fwd: y_planes %d", y_planes);
+  CDFO_REQUIRE(act >= 0 && act <= 2, CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_up2_fwd: act %d", act);
+  CDFO_REQUIRE(((uintptr_t)x8_1x & 15) == 0 && ((uintptr_t)wpk & 15) == 0 && ((uintptr_t)y & 15) == 0, CDFO_ERR_SHAPE,
+               "cdfo_conv3x3_pair_sm100_up2_fwd: pointers must be 16-byte aligned");
+  CDFO_REQUIRE(cpair::smem_bytes(Cin, 128, true) <= 227 * 1024, CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_up2_fwd: shared memory");
+  CUtensorMap tm;                // unused: the A operand is built from x8_1x, not loaded by TMA
+  memset(&tm, 0, sizeof(tm));
+  cpair::Params p;
+  p.wpk = (const uint8_t *)wpk; p.bias = bias; p.bias_edge = bias_edge; p.resid = nullptr; p.x1 = (const uint4 *)x8_1x; p.y = (uint4 *)y;
+  p.B = B; p.Cin = Cin; p.H = H2; p.W = W2; p.act = act; p.y_planes = y_planes; p.tma_wide = 0;
+  p.tiles_x = ceil_div(W2, cpair::kTileW); p.tiles_y = ceil_div(H2, cpair::kTileH);
+  const long long mt = (long long)B * p.tiles_x * p.tiles_y;
+  CDFO_REQUIRE(mt < (1ll << 30), CDFO_ERR_UNSUPPORTED, "cdfo_conv3x3_pair_sm100_up2_fwd: too many tiles");
+  p.m_tiles = (int)mt;
+  return cpair::launch<128, true>(tm, p, (cudaStream_t)stream);
 }

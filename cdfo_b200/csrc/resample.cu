@@ -6,29 +6,15 @@
 // clamped at 0 -> weights (0.25, 0.75) / (0.75, 0.25) with the edge pixel repeated.  One thread per output pixel and
 // 8-channel chunk (16 bytes in, 16 bytes out, fp32 arithmetic): pure HBM-bound kernels.
 #include "cdfo_common.cuh"
+#include "up2_blend.cuh"
 
 namespace cdfo {
 namespace rs {
 
-struct F8 { float v[8]; };
+using up2::F8;
+using up2::pack;
+using up2::unpack;
 
-__device__ __forceinline__ F8 unpack(const uint4 q) {
-  F8 r;
-  const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    r.v[2 * i] = __uint_as_float(w[i] << 16);
-    r.v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
-  }
-  return r;
-}
-__device__ __forceinline__ uint32_t bf2(float a, float b) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t *>(&v);
-}
-__device__ __forceinline__ uint4 pack(const F8 &a) {
-  return make_uint4(bf2(a.v[0], a.v[1]), bf2(a.v[2], a.v[3]), bf2(a.v[4], a.v[5]), bf2(a.v[6], a.v[7]));
-}
 __device__ __forceinline__ void axpy(F8 &acc, float w, const uint4 q) {
   const F8 t = unpack(q);
 #pragma unroll
@@ -100,20 +86,11 @@ __global__ void upsample2_c8_kernel(const uint4 *__restrict__ a, uint4 *__restri
   for (int k = 0; k < 3; ++k) {
     const uint4 *row = src + (size_t)rows[k] * Wi;
     const F8 xm = unpack(__ldg(row + jm)), x0 = unpack(__ldg(row + j)), xp = unpack(__ldg(row + jp));
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      l[k].v[c] = fmaf(0.25f, xm.v[c], 0.75f * x0.v[c]);
-      r[k].v[c] = fmaf(0.25f, xp.v[c], 0.75f * x0.v[c]);
-    }
+    l[k] = up2::blend(xm, x0);
+    r[k] = up2::blend(xp, x0);
   }
-  F8 o00, o01, o10, o11;               // rows 2i (0.25 row[i-1] + 0.75 row[i]) and 2i+1 (0.75 row[i] + 0.25 row[i+1])
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    o00.v[c] = fmaf(0.25f, l[0].v[c], 0.75f * l[1].v[c]);
-    o01.v[c] = fmaf(0.25f, r[0].v[c], 0.75f * r[1].v[c]);
-    o10.v[c] = fmaf(0.25f, l[2].v[c], 0.75f * l[1].v[c]);
-    o11.v[c] = fmaf(0.25f, r[2].v[c], 0.75f * r[1].v[c]);
-  }
+  // rows 2i (0.25 row[i-1] + 0.75 row[i]) and 2i+1 (0.75 row[i] + 0.25 row[i+1])
+  const F8 o00 = up2::blend(l[0], l[1]), o01 = up2::blend(r[0], r[1]), o10 = up2::blend(l[2], l[1]), o11 = up2::blend(r[2], r[1]);
   uint4 *d = y + (size_t)plane * 4 * Hi * Wi + (size_t)(2 * i) * (2 * Wi) + 2 * j;
   d[0] = pack(o00);
   d[1] = pack(o01);

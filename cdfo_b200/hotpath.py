@@ -436,7 +436,8 @@ def cross_scale_block(blk, x8, x8_half=None, want_half=False):
         wd0, bd0, ed0 = wts["body0_dn"]
         wu0, bu0, eu0 = wts["body0_up"]
         cu = conv.conv3x3(conv.conv3x3(xh, wd0, bd0, conv.ACT_LRELU, bias_edge=ed0), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
-        xu = conv.resample(x8, 1)
+        # config.trunk_fused_upsample: body.0 at 2x evaluates the bilinear x2 of x8 itself (no 2x input tensor in HBM)
+        xu = None if config.trunk_fused_upsample and config.conv_fold_half else conv.resample(x8, 1)
     else:
         xd = conv.conv3x3(xh, dn.weight, dn.bias, conv.ACT_NONE)            # 1x1
         cu = conv.conv3x3(conv.conv3x3(xd, b0.weight, b0.bias, conv.ACT_LRELU), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
@@ -444,7 +445,11 @@ def cross_scale_block(blk, x8, x8_half=None, want_half=False):
         wu0, bu0, eu0 = b0.weight, b0.bias, None
     if config.conv_fold_half:
         # the 2x-resolution intermediate lives as its four parity planes: the stride-2 taps of the folded convolution are dense boxes
-        t2 = conv.conv3x3(xu, wu0, bu0, conv.ACT_LRELU, parity_planes=config.conv_parity_planes and config.conv_pair, bias_edge=eu0)
+        planes = config.conv_parity_planes and config.conv_pair
+        if xu is None:
+            t2 = conv.conv3x3_up2(x8, wu0, bu0, conv.ACT_LRELU, parity_planes=planes, bias_edge=eu0)
+        else:
+            t2 = conv.conv3x3(xu, wu0, bu0, conv.ACT_LRELU, parity_planes=planes, bias_edge=eu0)
         # bilinear x0.5 of a 3x3 convolution = one 4x4 / stride-2 convolution: evaluated at 1x, the branch sum starts in its epilogue
         if fused:
             # ... and ends there: + bilinear x2 of the half-resolution branch, and the x0.5 of the sum for the next block's down branch

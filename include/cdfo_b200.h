@@ -309,6 +309,11 @@ int cdfo_conv3x3_pair_sm100_planes_fwd(const void *x_c8, const void *wpk, const 
  * followed by body.0, arch/SIDECVSR_our.py:388-406): its bias passes only under the taps that lie inside the frame. */
 int cdfo_conv3x3_pair_sm100_edge_fwd(const void *x_c8, const void *wpk, const float *bias, const float *bias_edge, const void *resid_c8,
                                      void *y, int B, int Cin, int Cout, int H, int W, int act, int y_planes, void *stream);
+/* The 64 -> 256 convolution applied to the bilinear x2 of x8_1x [B,8,H2/2,W2/2,8] bf16 (F.interpolate, align_corners=False) without
+ * materialising it: y = cdfo_conv3x3_pair_sm100_edge_fwd(cdfo_resample_c8(x8_1x, mode 1), ...) bit for bit, at the 2x size H2 x W2
+ * (both even).  Cin = 64, Cout = 256, no residual, y_planes 0 (c8) or 1 (parity planes); bias_edge may be NULL. */
+int cdfo_conv3x3_pair_sm100_up2_fwd(const void *x8_1x, const void *wpk, const float *bias, const float *bias_edge, void *y, int B, int Cin,
+                                    int Cout, int H2, int W2, int act, int y_planes, void *stream);
 /* ---- "3x3 convolution at 2H x 2W followed by bilinear x0.5" as ONE 4x4 / stride-2 convolution on a CTA pair
  * (csrc/conv4x4s2_pair_sm100.cu): the down(body(up(x))) branch of Block_.forward, arch/SIDECVSR_our.py:401-406 with Interpolate(0.5)
  * :324-333.  w3 [64,Cin,3,3] fp32 is the 3x3 weight (pack_weight folds the 2x2 mean into a 4x4 kernel);

@@ -60,6 +60,15 @@ struct LraTables {
 // csrc/lra_col_sm100.cu: tcgen05 column pass; 1 = launched, 0 = shape outside its limits (caller falls back), < 0 = error
 int lra_col_sm100_launch(const float *vrow_t, const uint8_t *midx, const float *qsel, float *long_out, const LraTables &t, int B, int H, int W,
                          cudaStream_t s);
+// host-only: whether lra_col_sm100_launch takes H rows (no CUDA call)
+bool lra_col_sm100_fits(int H);
+
+// csrc/dcn_tex_sm100.cu, csrc/mv_dcn_fused_sm100.cu: the x samples of a texture DCN call are bound as pitch-2D textures of at most
+// kTexRows rows (16 * (H + 3) rows per sample; fp32 texture coordinates keep >= 8 fractional bits below 65536 rows).  A call whose x batch
+// does not fit is split into the fewest slices of `per` consecutive samples (the last one may be shorter), one launch per slice.
+constexpr int kTexRows = 65000;
+struct TexSlices { int count, per; };
+TexSlices tex_slices(int x_batch, long long sample_rows);
 
 // csrc/pointwise.cu: tensor-core 1x1 convolution (see cdfo_pointwise_conv_fwd in include/cdfo_b200.h)
 int pointwise_conv(const float *in1, const float *in2, const float *w, const float *bias, const float *resid1, const float *resid2,

@@ -55,13 +55,14 @@ constexpr int kTmemCols = 256;        // [0,64) accumulator, [64,192) A operand 
 constexpr int kAColBase = 64, kAColsPerStage = 32;
 
 struct Params {
-  cudaTextureObject_t tex;           // ONE pitch-2D texture over all x samples: rows = (sample * 16 + quad) * (H + 3) + row
+  cudaTextureObject_t tex;           // ONE pitch-2D texture over the x samples [x0, x0 + xn): rows = ((sample - x0) * 16 + quad) * (H + 3) + row
   const uint2 *fields;               // [B][9 taps][dg/gp][H*W][gp] (dy, dx, m, 0) fp16, gp = 2 when dg = 16, else 1
   const float *mv;                   // [B][2][H*W] (x, y) or nullptr
   const uint8_t *wpk;                // [9][8][64][8] fp16
   const float *bias;
   void *y;
   int B, H, W, dg, out_mode, gshift, x_batch;
+  int x0, xn;                        // this launch's x slice: the tiles enumerate samples b = k * x_batch + j, j in [x0, x0 + xn)
   long long f_bstride;               // uint2 elements between samples of fields
   // c8 output placement: sample s goes to 8-channel chunks [(s % y_nb) * y_cs + y_grp[s / y_nb], +8) of y
   // (dense: y_nb = B, y_cs = 8, y_grp[0] = 0; stacked for tsa_fusion: y_nb = sequences, y_cs = 56, y_grp = frame slot * 8)
@@ -100,8 +101,9 @@ __device__ __forceinline__ uint2 ld_stream_u2(const uint2 *p) {
 struct TileCoord { int b, h0, w0; };
 __device__ __forceinline__ TileCoord tile_coord(const Params &p, int tile) {
   TileCoord t;
-  t.b = tile / p.tiles_per_img;
-  const int r = tile - t.b * p.tiles_per_img;
+  const int bl = tile / p.tiles_per_img;               // sample within this launch's x slice
+  const int r = tile - bl * p.tiles_per_img;
+  t.b = bl + (bl / p.xn) * (p.x_batch - p.xn) + p.x0;  // = bl when the slice is the whole x batch
   const int ty = r / p.tiles_x;
   t.h0 = ty * kTileH;
   t.w0 = (r - ty * p.tiles_x) * kTileW;
@@ -284,7 +286,7 @@ dcn_tex_sm100_kernel(const __grid_constant__ Params p, const __grid_constant__ C
       const int h = tc.h0 + ty, w = tc.w0 + tx;
       const int pixc = min(h, p.H - 1) * p.W + min(w, p.W - 1);
       s.f = p.fields + (size_t)tc.b * p.f_bstride + (kDG16 ? ((size_t)(quad0 >> 1) * P + pixc) * 2 : (size_t)pixc);
-      s.py = (float)(((tc.b % p.x_batch) * 16 + quad0) * (p.H + 3)) + 1.5f;
+      s.py = (float)(((tc.b % p.x_batch - p.x0) * 16 + quad0) * (p.H + 3)) + 1.5f;
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
         s.hb[i] = (float)(h - 1 + i);
@@ -492,6 +494,11 @@ static cudaError_t get_texture(const void *ptr, int rows, int W, int Wpt, cudaSt
 }  // namespace dtex
 
 // shared with csrc/mv_dcn_fused_sm100.cu
+TexSlices tex_slices(int x_batch, long long sample_rows) {
+  const int fit = (int)(kTexRows / sample_rows);        // >= 1: the callers reject taller frames
+  const int n = (x_batch + fit - 1) / fit;              // fewest slices that fit; equal sizes up to one sample
+  return TexSlices{n, (x_batch + n - 1) / n};
+}
 cudaError_t dcn_tex_get_texture(const void *ptr, int rows, int W, int Wpt, cudaStream_t stream, cudaTextureObject_t *out) {
   return dtex::get_texture(ptr, rows, W, Wpt, stream, out);
 }
@@ -560,15 +567,11 @@ static int dcn_tex_run(const void *x_q4t, const void *fields, const float *mv, c
   dtex::Params p;
   p.x_batch = x_batch > 0 ? x_batch : B;
   CDFO_REQUIRE(B % p.x_batch == 0, CDFO_ERR_SHAPE, "cdfo_dcn_tex_sm100_fwd: B (%d) must be a multiple of x_batch (%d)", B, p.x_batch);
-  // one texture over all x samples; fp32 texture coordinates keep >= 8 fractional bits (the filter's resolution) below 65536 rows
-  CDFO_REQUIRE((long long)p.x_batch * 16 * (H + 3) <= 65000, CDFO_ERR_UNSUPPORTED,
-               "cdfo_dcn_tex_sm100_fwd: x_batch * 16 * (H + 3) = %lld rows exceed the 2-D linear texture limit (65000): split the call",
-               (long long)p.x_batch * 16 * (H + 3));
+  // one texture per x slice; fp32 texture coordinates keep >= 8 fractional bits (the filter's resolution) below 65536 rows
+  const long long sample_rows = 16ll * (H + 3);
+  CDFO_REQUIRE(sample_rows <= kTexRows, CDFO_ERR_UNSUPPORTED,
+               "cdfo_dcn_tex_sm100_fwd: frame height %d exceeds the 2-D linear texture limit (16 * (H + 3) <= %d rows)", H, kTexRows);
   const int Wpt = cdfo_q4t_pitch(W);
-  {
-    cudaError_t e = dtex::get_texture(x_q4t, p.x_batch * 16 * (H + 3), W, Wpt, (cudaStream_t)stream, &p.tex);
-    if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cdfo_dcn_tex_sm100_fwd: cudaCreateTextureObject: %s", cudaGetErrorString(e));
-  }
   p.fields = (const uint2 *)fields; p.mv = mv; p.wpk = (const uint8_t *)wpk; p.bias = bias; p.y = y;
   p.B = B; p.H = H; p.W = W; p.dg = dg; p.out_mode = out_mode;
   p.y_nb = y_nb; p.y_cs = y_cs;
@@ -581,9 +584,6 @@ static int dcn_tex_run(const void *x_q4t, const void *fields, const float *mv, c
   CDFO_REQUIRE((long long)dg * 9 * H * W < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_dcn_tex_sm100_fwd: field planes too large for 32-bit indexing");
   const long long nt = (long long)p.tiles_per_img * B;
   CDFO_REQUIRE(nt < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_dcn_tex_sm100_fwd: too many tiles");
-  p.num_tiles = (int)nt;
-  int grid = num_ctas > 0 ? num_ctas : kNumSMs;
-  if (grid > p.num_tiles) grid = p.num_tiles;
   // mode 2 (fields through TMA) needs the dense [B][9][8][H][W][2] layout; tiny frames keep the LDG path
   const bool dense = p.f_bstride == (long long)dg * 9 * H * W;
   int mode = dg != 16 ? 0 : (dense && W >= dtex::kTileW && H >= dtex::kTileH && !dtex::g_no_tma_fields ? 2 : 1);
@@ -614,8 +614,20 @@ static int dcn_tex_run(const void *x_q4t, const void *fields, const float *mv, c
   }
   const int threads = (dtex::kEpiWarps + dtex::kProdWarps) * 32;
   cudaStream_t st = (cudaStream_t)stream;
-  if (mode == 2) dtex::dcn_tex_sm100_kernel<2><<<grid, threads, dtex::smem_bytes(2), st>>>(p, ftm);
-  else if (mode == 1) dtex::dcn_tex_sm100_kernel<1><<<grid, threads, dtex::smem_bytes(1), st>>>(p, ftm);
-  else dtex::dcn_tex_sm100_kernel<0><<<grid, threads, dtex::smem_bytes(0), st>>>(p, ftm);
-  return check_launch("cdfo_dcn_tex_sm100_fwd");
+  const TexSlices sl = tex_slices(p.x_batch, sample_rows);
+  for (int x0 = 0; x0 < p.x_batch; x0 += sl.per) {
+    p.x0 = x0;
+    p.xn = p.x_batch - x0 < sl.per ? p.x_batch - x0 : sl.per;
+    const uint8_t *base = (const uint8_t *)x_q4t + (size_t)x0 * (size_t)sample_rows * Wpt * 8;   // a multiple of 512 bytes
+    cudaError_t e = dtex::get_texture(base, (int)(p.xn * sample_rows), W, Wpt, st, &p.tex);
+    if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cdfo_dcn_tex_sm100_fwd: cudaCreateTextureObject: %s", cudaGetErrorString(e));
+    p.num_tiles = p.tiles_per_img * (B / p.x_batch) * p.xn;
+    int grid = num_ctas > 0 ? num_ctas : kNumSMs;
+    if (grid > p.num_tiles) grid = p.num_tiles;
+    if (mode == 2) dtex::dcn_tex_sm100_kernel<2><<<grid, threads, dtex::smem_bytes(2), st>>>(p, ftm);
+    else if (mode == 1) dtex::dcn_tex_sm100_kernel<1><<<grid, threads, dtex::smem_bytes(1), st>>>(p, ftm);
+    else dtex::dcn_tex_sm100_kernel<0><<<grid, threads, dtex::smem_bytes(0), st>>>(p, ftm);
+    if (int rc = check_launch("cdfo_dcn_tex_sm100_fwd")) return rc;
+  }
+  return CDFO_OK;
 }

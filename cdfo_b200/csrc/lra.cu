@@ -129,17 +129,40 @@ constexpr int kRowWarps = 9, kRowThreads = kRowWarps * 32;
 // element (32 768 per row: two thirds of the kernel, ncu + the same finding as csrc/lra_mask_logits.cu).  Same fp32 operation order.
 constexpr int kRowPiece = 64;
 constexpr int kRowRawBytes = 2 * 64 * kRowPiece * 4 + 64;      // two pieces + four mbarriers (128-byte aligned in front of vr)
-template <bool TMA>
+// NCTA > 1 (rows too wide for one CTA's shared memory): the row is split over a cluster of NCTA CTAs (NCTA, 1, 1).  CTA rank r holds vr
+// only for its slice [r * Ws, r * Ws + Ws) of the keys (whole 64-key blocks) and owns the queries of the same columns; the small per-key
+// arrays, m0 and d0 cover the whole row in every CTA.  The N0 partials over each slice are exchanged through distributed shared memory and
+// summed in rank order; a masked query's flash tile reads the key blocks of other slices from the holder's shared memory (generic loads
+// through mapa addresses).  NCTA = 1 is the single-CTA kernel: every NCTA branch below folds away at compile time.
+__host__ __device__ constexpr int lra_row_slice(int Wk, int ncta) { return ((Wk / 64 + ncta - 1) / ncta) * 64; }
+
+template <typename T>
+__device__ __forceinline__ const T *peer_smem(const T *p, int rank) {   // generic address of the same shared-memory offset in CTA `rank`
+  uint64_t r;
+  asm volatile("mapa.u64 %0, %1, %2;" : "=l"(r) : "l"(p), "r"(rank));
+  return reinterpret_cast<const T *>(r);
+}
+__device__ __forceinline__ void row_cluster_sync() {
+  __syncwarp();
+  asm volatile("barrier.cluster.arrive.release;\n\tbarrier.cluster.wait.acquire;" ::: "memory");
+}
+
+template <int NCTA, bool TMA>
 __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_constant__ CUtensorMap qvmap, const float *__restrict__ qv,
                                                                 const uint8_t *__restrict__ midx, const float *__restrict__ qsel,
                                                                 float *__restrict__ vrow_t, LraTables t, int H, int W) {
   extern __shared__ __align__(1024) float sm_all[];
   float *sm = TMA ? sm_all + kRowRawBytes / 4 : sm_all;
-  const int b = blockIdx.y, h = blockIdx.x;
+  const int b = blockIdx.y, h = blockIdx.x / NCTA;
+  const int rank = NCTA == 1 ? 0 : (int)(blockIdx.x % NCTA);   // = %cluster_ctarank for cluster dims (NCTA, 1, 1)
   const int HW = H * W;
   const int Wk = (W + 63) & ~63;      // keys padded to whole 64-key blocks
-  float *vr = sm;                     // [Wk][kLd] conv1x9(v) as TF32 bits (rows >= W zero)
-  float *Rs = vr + Wk * kLd;          // [64*64] R table
+  const int Ws = NCTA == 1 ? Wk : lra_row_slice(Wk, NCTA);
+  const int k_lo = rank * Ws;                                  // this CTA's keys [k_lo, k_hi) and queries [k_lo, w_end)
+  const int k_hi = NCTA == 1 ? Wk : min(k_lo + Ws, Wk);
+  const int w_end = NCTA == 1 ? W : min(W, k_hi);
+  float *vr = sm;                     // [Ws][kLd] conv1x9(v) of keys k_lo + row as TF32 bits (keys >= W zero)
+  float *Rs = vr + Ws * kLd;          // [64*64] R table
   float *sw = Rs + 4096;              // [Wk]  beta * s_w
   float *e0 = sw + Wk;                // [Wk]  exp(beta s_w - m0)
   float *qs = e0 + Wk;                // [Wk]  q of the masked channel
@@ -168,20 +191,20 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
       ptx::fence_mbar_init();
     }
     __syncthreads();
-    const int n_pieces = Wk / kRowPiece;
+    const int n_pieces = (k_hi - k_lo) / kRowPiece;
     if (warp == 8) {
       if (lane == 0) {
         for (int pc = 0; pc < n_pieces; ++pc) {
           const int st = pc & 1;
           ptx::mbar_wait_parked(bar0 + 16 + 8 * st, ((pc >> 1) & 1) ^ 1);
           ptx::mbar_arrive_expect_tx(bar0 + 8 * st, 64 * kRowPiece * 4);
-          ptx::tma_load_3d(ptx::smem_u32(raw) + st * 64 * kRowPiece * 4, &qvmap, bar0 + 8 * st, pc * kRowPiece, h, b * 128 + 64);
+          ptx::tma_load_3d(ptx::smem_u32(raw) + st * 64 * kRowPiece * 4, &qvmap, bar0 + 8 * st, k_lo + pc * kRowPiece, h, b * 128 + 64);
         }
       }
     } else {
       const int px = tid & 63, c0 = (tid >> 6) * 16;                        // 256 threads: pixel x quarter of the channels
       for (int pc = 0; pc < n_pieces; ++pc) {
-        const int st = pc & 1, w = pc * kRowPiece + px;
+        const int st = pc & 1, w = k_lo + pc * kRowPiece + px;
         ptx::mbar_wait_parked(bar0 + 8 * st, (pc >> 1) & 1);
         const float *rp = raw + st * 64 * kRowPiece + px;
         float win[24];                                                      // channels c0 - 4 .. c0 + 19 (zero outside 0 .. 63)
@@ -192,7 +215,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
         }
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(bar0 + 16 + 8 * st);                // the piece is in registers
-        float *row = vr + w * kLd + c0;
+        float *row = vr + (w - k_lo) * kLd + c0;
 #pragma unroll
         for (int c4 = 0; c4 < 4; ++c4) {
           float o[4];
@@ -213,10 +236,11 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
   const float *vbase = qv + ((size_t)b * 128 + 64) * HW + (size_t)h * W;
   // (4-byte cp.async: the ~107 copies of a thread are all in flight at once -- with one CTA of 9 warps per SM a load -> store loop
   // through registers leaves the SM waiting on one DRAM round trip per iteration)
-  for (int e = tid; e < 64 * Wk; e += kRowThreads) {
-    const int c = e / Wk, w = e - c * Wk;
+  const int Wn = k_hi - k_lo;
+  for (int e = tid; e < 64 * Wn; e += kRowThreads) {
+    const int c = e / Wn, wl = e - c * Wn, w = k_lo + wl;
     const bool ok = w < W;
-    const uint32_t dst = (uint32_t)__cvta_generic_to_shared(vr + w * kLd + c);
+    const uint32_t dst = (uint32_t)__cvta_generic_to_shared(vr + wl * kLd + c);
     const float *src = vbase + (size_t)c * HW + (ok ? w : 0);
     const int nb = ok ? 4 : 0;            // src-size 0: zero fill
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(src), "r"(nb) : "memory");
@@ -224,7 +248,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
   asm volatile("cp.async.commit_group;" ::: "memory");
   asm volatile("cp.async.wait_group 0;" ::: "memory");
   __syncthreads();
-  for (int w = tid; w < W; w += kRowThreads) {
+  for (int w = tid; w < w_end - k_lo; w += kRowThreads) {
     float *row = vr + w * kLd;
     float win[72];                         // channels -4 .. 67 of this pixel (zero outside 0 .. 63)
 #pragma unroll
@@ -261,7 +285,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
     cs[w] = on ? c : -1;
     qs[w] = q;
     sw[w] = on ? t.beta * q * t.k1[c] : 0.f;
-    if (on) mlist[atomicAdd(&mcount, 1)] = w;
+    if (on && (NCTA == 1 || (w >= k_lo && w < k_hi))) mlist[atomicAdd(&mcount, 1)] = w;
   }
   __syncthreads();
   // common distribution of every unmasked query: softmax_w'(beta * s_w')
@@ -296,22 +320,41 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
     const int c = tid & 63, part = tid >> 6;
     float acc = 0.f;
     if (part < 4)
-      for (int w = part; w < W; w += 4) acc = fmaf(e0[w], vr[w * kLd + c], acc);
+      for (int w = k_lo + part; w < w_end; w += 4) acc = fmaf(e0[w], vr[(w - k_lo) * kLd + c], acc);
     __syncthreads();
     red[tid] = acc;
     __syncthreads();
-    if (tid < 64) n0[tid] = (red[tid] + red[tid + 64] + red[tid + 128] + red[tid + 192]) / d0_s;
+    if (NCTA == 1) {
+      if (tid < 64) n0[tid] = (red[tid] + red[tid + 64] + red[tid + 128] + red[tid + 192]) / d0_s;
+    } else {
+      if (tid < 64) red[tid] = red[tid] + red[tid + 64] + red[tid + 128] + red[tid + 192];   // this slice's partial, read by every peer
+    }
+  }
+  if (NCTA > 1) {
+    // round this slice's v_r to TF32 here: the cluster barrier below then publishes both the partials and the finished key blocks
+    for (int e = tid; e < (k_hi - k_lo) * 64; e += kRowThreads) {
+      float *p = vr + (e >> 6) * kLd + (e & 63);
+      *p = __uint_as_float(to_tf32(*p));
+    }
+    row_cluster_sync();
+    if (tid < 64) {
+      float s = 0.f;
+      for (int r = 0; r < NCTA; ++r) s += r == rank ? red[tid] : peer_smem(red, r)[tid];   // rank order: the same sum in every CTA
+      n0[tid] = s / d0_s;
+    }
   }
   __syncthreads();
   // unmasked queries: the common vector
-  for (int e = tid; e < W * 64; e += kRowThreads) {
+  for (int e = k_lo * 64 + tid; e < w_end * 64; e += kRowThreads) {
     const int w = e >> 6, c = e & 63;
     if (cs[w] < 0) vrow_t[(((size_t)b * W + w) * H + h) * 64 + c] = n0[c];
   }
-  // round v_r to TF32 in place for the tensor-core pass
-  for (int e = tid; e < Wk * 64; e += kRowThreads) {
-    float *p = vr + (e >> 6) * kLd + (e & 63);
-    *p = __uint_as_float(to_tf32(*p));
+  if (NCTA == 1) {
+    // round v_r to TF32 in place for the tensor-core pass
+    for (int e = tid; e < Wk * 64; e += kRowThreads) {
+      float *p = vr + (e >> 6) * kLd + (e & 63);
+      *p = __uint_as_float(to_tf32(*p));
+    }
   }
   __syncthreads();
   // masked queries: own softmax over w'; one warp per tile of 16 masked queries
@@ -346,7 +389,12 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
           sc[n][2 * r + 1] = c2.y >= 0 ? fmaf(q1[r] * q2.y, Rs[c1[r] * 64 + c2.y], s2.y) : s2.y;
         }
       }
-      flash_tile_block(sc, m_run, l_run, o, Vu, key0, W, g, tq);
+      if (NCTA == 1) {
+        flash_tile_block(sc, m_run, l_run, o, Vu, key0, W, g, tq);
+      } else {   // the block's holder, with keys counted from the start of its slice
+        const int r = key0 / Ws, lo = r * Ws;
+        flash_tile_block(sc, m_run, l_run, o, r == rank ? Vu : peer_smem(Vu, r), key0 - lo, W - lo, g, tq);
+      }
     }
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
@@ -362,6 +410,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) lra_row_kernel(const __grid_co
       for (int n = 0; n < 8; ++n) *reinterpret_cast<float2 *>(dst + 8 * n) = make_float2(o[n][2 * r] * inv, o[n][2 * r + 1] * inv);
     }
   }
+  if (NCTA > 1) row_cluster_sync();   // no CTA retires while a peer may still read its key blocks
 }
 
 // ------------------------------------------------------------------------------------------------ flash-style block
@@ -983,6 +1032,32 @@ static int lra_run(const float *qv, const float *u, const float *vmax, const flo
   CDFO_REQUIRE(qv && u && vmax && x && tables && fuse_w && fuse_b && (out || out_c8) && workspace, CDFO_ERR_NULL, "cdfo_lra_fwd: NULL pointer");
   CDFO_REQUIRE(B > 0 && B <= 65535 && H > 0 && W > 0 && H % 8 == 0 && W % 8 == 0, CDFO_ERR_SHAPE,
                "cdfo_lra_fwd: H and W must be multiples of the window size 8 (got %d x %d)", H, W);
+  // every shape check comes before the first launch: a rejected call leaves the workspace untouched
+  const int kDynMax = 224 * 1024;  // 227 KB opt-in limit minus the kernels' small static shared memory
+  const int Wk = (W + 63) & ~63;
+  auto row_bytes = [&](int ncta) {   // the row kernel's dynamic shared memory (without the TMA ring) when ncta CTAs share a row
+    const size_t Ws = ncta == 1 ? (size_t)Wk : (size_t)lra_row_slice(Wk, ncta);
+    return (Ws * kLd + 4096 + 3 * (size_t)Wk + 64 + kRowThreads + 2 * (size_t)Wk) * 4;
+  };
+  const int row_ncta = row_bytes(1) <= (size_t)kDynMax ? 1 : 2;   // by width alone: W <= 704 runs on one CTA
+  const size_t row_smem = row_bytes(row_ncta);
+  const int Hk = (H + 63) & ~63;
+  const size_t col_v = (size_t)Hk * kLd > (size_t)(H + 8) * 64 ? (size_t)Hk * kLd : (size_t)(H + 8) * 64;
+  const size_t col_smem = ((size_t)Hk * kLd + col_v) * 4;
+  const size_t col16_smem = ((size_t)Hk * kQw + 64 * ((size_t)Hk / 2 + 4) + 2 * (size_t)(H + 8) + 16) * 4;
+  const size_t win_smem = (size_t)3 * 64 * kLd * 4;
+  CDFO_REQUIRE(row_smem <= (size_t)kDynMax, CDFO_ERR_UNSUPPORTED,
+               "cdfo_lra_fwd: frame width %d exceeds the row pass's shared memory over a 2-CTA cluster (W <= 1280)", W);
+  // the column kernel that will run: tcgen05 when it takes the shape, else the bf16 mma.sync kernel; the TF32 one only on request
+  const bool col_tc = !g_lra_col_tf32 && g_lra_col_tc && lra_col_sm100_fits(H);
+  if (!col_tc) {
+    if (g_lra_col_tf32)
+      CDFO_REQUIRE(col_smem <= (size_t)kDynMax, CDFO_ERR_UNSUPPORTED,
+                   "cdfo_lra_fwd: frame height %d exceeds the TF32 column pass's shared memory (H <= 384)", H);
+    else
+      CDFO_REQUIRE(col16_smem <= (size_t)kDynMax, CDFO_ERR_UNSUPPORTED,
+                   "cdfo_lra_fwd: frame height %d exceeds the bf16 column pass's shared memory (H <= 768)", H);
+  }
   cudaStream_t s = (cudaStream_t)stream;
   const size_t P = (size_t)B * H * W;
   const int HW = H * W;
@@ -993,22 +1068,12 @@ static int lra_run(const float *qv, const float *u, const float *vmax, const flo
   float *loc_out = long_out + P * 64;
   uint8_t *midx = (uint8_t *)(loc_out + P * 64);
   LraTables t{tables, tables + 9, tables + 18, tables + 82, beta, bh};
-
-  lra_mask_kernel<<<dim3(ceil_div(HW, 128), B), 128, 0, s>>>(u, vmax, qv, midx, qsel, HW);
-
-  const int Wk = (W + 63) & ~63;
-  const size_t row_smem = ((size_t)Wk * kLd + 4096 + 3 * (size_t)Wk + 64 + kRowThreads + 2 * (size_t)Wk) * 4;
-  const int Hk = (H + 63) & ~63;
-  const size_t col_v = (size_t)Hk * kLd > (size_t)(H + 8) * 64 ? (size_t)Hk * kLd : (size_t)(H + 8) * 64;
-  const size_t col_smem = ((size_t)Hk * kLd + col_v) * 4;
-  const size_t win_smem = (size_t)3 * 64 * kLd * 4;
-  const int kDynMax = 224 * 1024;  // 227 KB opt-in limit minus the kernels' small static shared memory
-  CDFO_REQUIRE(row_smem <= (size_t)kDynMax && col_smem <= (size_t)kDynMax, CDFO_ERR_UNSUPPORTED,
-               "cdfo_lra_fwd: frame %d x %d exceeds the shared-memory row/column buffers (W <= 704, H <= 384)", H, W);
   static bool attr = false;
   if (!attr) {
-    cudaError_t e1 = cudaFuncSetAttribute(lra_row_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
-    if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(lra_row_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
+    cudaError_t e1 = cudaFuncSetAttribute(lra_row_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
+    if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(lra_row_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
+    if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(lra_row_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
+    if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(lra_row_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
     cudaError_t e2 = cudaFuncSetAttribute(lra_col_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
     if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(lra_col_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynMax);
     cudaError_t e3 = cudaFuncSetAttribute(lra_win_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_smem);
@@ -1016,6 +1081,9 @@ static int lra_run(const float *qv, const float *u, const float *vmax, const flo
       return fail(CDFO_ERR_CUDA, "cdfo_lra_fwd: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : (e2 != cudaSuccess ? e2 : e3)));
     attr = true;
   }
+
+  lra_mask_kernel<<<dim3(ceil_div(HW, 128), B), 128, 0, s>>>(u, vmax, qv, midx, qsel, HW);
+
   {
     CUtensorMap qm;
     memset(&qm, 0, sizeof(qm));
@@ -1034,19 +1102,34 @@ static int lra_run(const float *qv, const float *u, const float *vmax, const flo
         row_tma = false;
       }
     }
-    if (row_tma) lra_row_kernel<true><<<dim3(H, B), kRowThreads, row_smem + kRowRawBytes, s>>>(qm, qv, midx, qsel, vrow_t, t, H, W);
-    else lra_row_kernel<false><<<dim3(H, B), kRowThreads, row_smem, s>>>(qm, qv, midx, qsel, vrow_t, t, H, W);
+    const size_t row_dyn = row_smem + (row_tma ? kRowRawBytes : 0);
+    if (row_ncta == 1) {
+      if (row_tma) lra_row_kernel<1, true><<<dim3(H, B), kRowThreads, row_dyn, s>>>(qm, qv, midx, qsel, vrow_t, t, H, W);
+      else lra_row_kernel<1, false><<<dim3(H, B), kRowThreads, row_dyn, s>>>(qm, qv, midx, qsel, vrow_t, t, H, W);
+    } else {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(2 * H, B);
+      cfg.blockDim = dim3(kRowThreads);
+      cfg.dynamicSmemBytes = row_dyn;
+      cfg.stream = s;
+      cudaLaunchAttribute at[1];
+      at[0].id = cudaLaunchAttributeClusterDimension;
+      at[0].val.clusterDim.x = 2;
+      at[0].val.clusterDim.y = 1;
+      at[0].val.clusterDim.z = 1;
+      cfg.attrs = at;
+      cfg.numAttrs = 1;
+      const cudaError_t e = row_tma ? cudaLaunchKernelEx(&cfg, lra_row_kernel<2, true>, qm, qv, midx, qsel, vrow_t, t, H, W)
+                                    : cudaLaunchKernelEx(&cfg, lra_row_kernel<2, false>, qm, qv, midx, qsel, vrow_t, t, H, W);
+      if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cdfo_lra_fwd: cluster launch of the row pass: %s", cudaGetErrorString(e));
+    }
   }
-  int col_done = 0;
-  if (!g_lra_col_tf32 && g_lra_col_tc) {     // csrc/lra_col_sm100.cu: whole score tile in tensor memory (H <= 448)
-    col_done = lra_col_sm100_launch(vrow_t, midx, qsel, long_out, t, B, H, W, s);
-    if (col_done < 0) return col_done;
-  }
-  if (col_done) {
+  if (col_tc) {     // csrc/lra_col_sm100.cu: whole score tile in tensor memory (H <= 384)
+    const int rc = lra_col_sm100_launch(vrow_t, midx, qsel, long_out, t, B, H, W, s);
+    if (rc < 0) return rc;
   } else if (g_lra_col_tf32) {
     lra_col_kernel<<<dim3(W, B), kColThreads, col_smem, s>>>(vrow_t, midx, qsel, long_out, t, H, W);
   } else {
-    const size_t col16_smem = ((size_t)Hk * kQw + 64 * ((size_t)Hk / 2 + 4) + 2 * (size_t)(H + 8) + 16) * 4;
     lra_col_bf16_kernel<<<dim3(W, B), kColThreads, col16_smem, s>>>(vrow_t, midx, qsel, long_out, t, H, W);
   }
   if (g_lra_win_tc) lra_win_tc_kernel<<<dim3(W / 8, H / 8, B), kWinTcThreads, 0, s>>>(qv, midx, loc_out, H, W);

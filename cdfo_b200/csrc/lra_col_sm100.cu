@@ -357,19 +357,29 @@ __global__ void __launch_bounds__(kThreads, 1) lra_col_sm100_kernel(const Params
 
 }  // namespace lct
 
+// dynamic shared memory of the kernel for H rows, 0 if the shape is outside its limits
+static size_t lra_col_sm100_smem(int H) {
+  const int Hp = (H + 15) & ~15;
+  if (Hp > 448) return 0;
+  const int Mp = ceil_div(H, 128) * 128 > Hp ? ceil_div(H, 128) * 128 : Hp;
+  const size_t smem = 2 * ((size_t)Mp * 128 + (size_t)Hp * 128) + (((size_t)(2 * (H + 8) + 16) * 4 + 15) & ~(size_t)15) + 8 * 8 + 16;
+  return smem > 227 * 1024 ? 0 : smem;
+}
+
+bool lra_col_sm100_fits(int H) { return lra_col_sm100_smem(H) != 0; }
+
 // returns 1 if the kernel was launched, 0 if the shape is outside its limits (the caller falls back to the mma.sync kernel), < 0 on error
 int lra_col_sm100_launch(const float *vrow_t, const uint8_t *midx, const float *qsel, float *long_out, const LraTables &t, int B, int H, int W,
                          cudaStream_t s) {
+  const size_t smem = lra_col_sm100_smem(H);
+  if (!smem) return 0;
   const int Hp = (H + 15) & ~15;
-  if (Hp > 448) return 0;
   lct::Params p;
   p.vrow_t = vrow_t; p.midx = midx; p.qsel = qsel; p.long_out = long_out; p.t = t;
   p.B = B; p.H = H; p.W = W; p.Hp = Hp;
   p.n_mt = ceil_div(H, 128);
   p.Mp = p.n_mt * 128 > Hp ? p.n_mt * 128 : Hp;
   p.ncols = B * W;
-  const size_t smem = 2 * ((size_t)p.Mp * 128 + (size_t)Hp * 128) + (((size_t)(2 * (H + 8) + 16) * 4 + 15) & ~(size_t)15) + 8 * 8 + 16;
-  if (smem > 227 * 1024) return 0;
   static size_t attr_smem = 0;
   if (smem > attr_smem) {
     cudaError_t e = cudaFuncSetAttribute(lct::lra_col_sm100_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

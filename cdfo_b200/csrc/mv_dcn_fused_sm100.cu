@@ -65,7 +65,7 @@ constexpr int kBarZFull = 0, kBarZEmpty = 2, kBarWFull = 4, kBarWEmpty = 7, kBar
               kBarAEmpty = 16, kBarDFull = 20, kBarDEmpty = 21, kBarDcnW = 22;
 
 struct Params {
-  cudaTextureObject_t tex;   // pitch-2D texture over all x samples (q4t), rows = (sample * 16 + quad) * (H + 3) + row
+  cudaTextureObject_t tex;   // pitch-2D texture over the x samples [x0, x0 + xn) (q4t), rows = ((sample - x0) * 16 + quad) * (H + 3) + row
   const uint8_t *hw;         // head weights [3 triples][9 head taps][8 chunks][144][8] bf16, channels permuted (see host side)
   const float *hbias;        // [432] permuted the same way
   const float *mv;           // [B][2][H*W] (x, y) or nullptr
@@ -75,6 +75,7 @@ struct Params {
   uint2 *fields_out;         // debug tap: the fields this kernel computed, [B][9][8][H*W][2] x (dy, dx | m, 0) fp16, or nullptr
   float mag;
   int B, H, W, out_mode, x_batch;
+  int x0, xn;                // this launch's x slice (csrc/dcn_tex_sm100.cu)
   int y_nb, y_cs, y_grp[8];  // c8 placement, as in dcn_tex_sm100.cu
   int tiles_x, tiles_per_img, num_tiles;
   int poll_ns;               // back-off between failed probes of the producers' long waits (0: none)
@@ -83,8 +84,9 @@ struct Params {
 struct TileCoord { int b, h0, w0; };
 __device__ __forceinline__ TileCoord tile_coord(const Params &p, int tile) {
   TileCoord t;
-  t.b = tile / p.tiles_per_img;
-  const int r = tile - t.b * p.tiles_per_img;
+  const int bl = tile / p.tiles_per_img;               // sample within this launch's x slice
+  const int r = tile - bl * p.tiles_per_img;
+  t.b = bl + (bl / p.xn) * (p.x_batch - p.xn) + p.x0;  // = bl when the slice is the whole x batch
   const int ty = r / p.tiles_x;
   t.h0 = ty * kTileH;
   t.w0 = (r - ty * p.tiles_x) * kTileW;
@@ -327,7 +329,7 @@ mv_head_dcn_fused_sm100_kernel(const __grid_constant__ Params p, const __grid_co
       const int pixc = min(h, p.H - 1) * p.W + min(w, p.W - 1);
       const float mvx = p.mv ? __ldg(p.mv + ((size_t)tc.b * 2 + 0) * P + pixc) : 0.f;
       const float mvy = p.mv ? __ldg(p.mv + ((size_t)tc.b * 2 + 1) * P + pixc) : 0.f;
-      const float py = (float)(((tc.b % p.x_batch) * 16 + qs * 4) * plane_rows) + 1.5f;   // texture row of image row -1.5, first quad
+      const float py = (float)(((tc.b % p.x_batch - p.x0) * 16 + qs * 4) * plane_rows) + 1.5f;   // texture row of image row -1.5, first quad
       const float wb0 = (float)(w - 1) + 1.5f;                                              // border shift + texel centre
 #pragma unroll
       for (int T = 0; T < 3; ++T) {
@@ -447,15 +449,11 @@ static int run(const void *z_c8, const void *head_wpk, const float *head_bias, f
   memset(&p, 0, sizeof(p));
   p.x_batch = x_batch > 0 ? x_batch : B;
   CDFO_REQUIRE(B % p.x_batch == 0, CDFO_ERR_SHAPE, "cdfo_mv_head_dcn_fused_sm100_fwd: B (%d) must be a multiple of x_batch (%d)", B, p.x_batch);
-  CDFO_REQUIRE((long long)p.x_batch * 16 * (H + 3) <= 65000, CDFO_ERR_UNSUPPORTED,
-               "cdfo_mv_head_dcn_fused_sm100_fwd: x_batch * 16 * (H + 3) = %lld rows exceed the 2-D linear texture limit (65000): split the call",
-               (long long)p.x_batch * 16 * (H + 3));
+  const long long sample_rows = 16ll * (H + 3);
+  CDFO_REQUIRE(sample_rows <= kTexRows, CDFO_ERR_UNSUPPORTED,
+               "cdfo_mv_head_dcn_fused_sm100_fwd: frame height %d exceeds the 2-D linear texture limit (16 * (H + 3) <= %d rows)", H, kTexRows);
   CDFO_REQUIRE((long long)9 * 16 * H * W < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_mv_head_dcn_fused_sm100_fwd: frame too large for 32-bit indexing");
   const int Wpt = cdfo_q4t_pitch(W);
-  {
-    cudaError_t e = dcn_tex_get_texture(x_q4t, p.x_batch * 16 * (H + 3), W, Wpt, (cudaStream_t)stream, &p.tex);
-    if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cdfo_mv_head_dcn_fused_sm100_fwd: cudaCreateTextureObject: %s", cudaGetErrorString(e));
-  }
   fdcn::EncodeTiledFn enc = fdcn::encode_tiled_fn();
   CDFO_REQUIRE(enc, CDFO_ERR_CUDA, "cdfo_mv_head_dcn_fused_sm100_fwd: cuTensorMapEncodeTiled not available from the driver");
   // hidden maps: c8 bf16 [2 B][8][H][W][8]; pixel and channel axes merged so that TMA issues one request per halo row
@@ -476,21 +474,30 @@ static int run(const void *z_c8, const void *head_wpk, const float *head_bias, f
   p.tiles_per_img = p.tiles_x * ceil_div(H, fdcn::kTileH);
   const long long nt = (long long)p.tiles_per_img * B;
   CDFO_REQUIRE(nt < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_mv_head_dcn_fused_sm100_fwd: too many tiles");
-  p.num_tiles = (int)nt;
   {
     static const int poll = getenv("CDFO_FUSED_POLL_NS") ? atoi(getenv("CDFO_FUSED_POLL_NS")) : 0;
     p.poll_ns = poll;
   }
-  int grid = num_ctas > 0 ? num_ctas : kNumSMs;
-  if (grid > p.num_tiles) grid = p.num_tiles;
   static bool attr_done = false;
   if (!attr_done) {
     cudaError_t e = cudaFuncSetAttribute(fdcn::mv_head_dcn_fused_sm100_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fdcn::kSmemBytes);
     if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cudaFuncSetAttribute(mv_head_dcn_fused_sm100): %s", cudaGetErrorString(e));
     attr_done = true;
   }
-  fdcn::mv_head_dcn_fused_sm100_kernel<<<grid, fdcn::kThreads, fdcn::kSmemBytes, (cudaStream_t)stream>>>(p, ztm);
-  return check_launch("cdfo_mv_head_dcn_fused_sm100_fwd");
+  const TexSlices sl = tex_slices(p.x_batch, sample_rows);
+  for (int x0 = 0; x0 < p.x_batch; x0 += sl.per) {
+    p.x0 = x0;
+    p.xn = p.x_batch - x0 < sl.per ? p.x_batch - x0 : sl.per;
+    const uint8_t *base = (const uint8_t *)x_q4t + (size_t)x0 * (size_t)sample_rows * Wpt * 8;   // a multiple of 512 bytes
+    cudaError_t e = dcn_tex_get_texture(base, (int)(p.xn * sample_rows), W, Wpt, (cudaStream_t)stream, &p.tex);
+    if (e != cudaSuccess) return fail(CDFO_ERR_CUDA, "cdfo_mv_head_dcn_fused_sm100_fwd: cudaCreateTextureObject: %s", cudaGetErrorString(e));
+    p.num_tiles = p.tiles_per_img * (B / p.x_batch) * p.xn;
+    int grid = num_ctas > 0 ? num_ctas : kNumSMs;
+    if (grid > p.num_tiles) grid = p.num_tiles;
+    fdcn::mv_head_dcn_fused_sm100_kernel<<<grid, fdcn::kThreads, fdcn::kSmemBytes, (cudaStream_t)stream>>>(p, ztm);
+    if (int rc = check_launch("cdfo_mv_head_dcn_fused_sm100_fwd")) return rc;
+  }
+  return CDFO_OK;
 }
 
 }  // namespace fdcn

@@ -132,7 +132,9 @@ int cdfo_pack_q4p(const float *x_nchw, void *x_q4p, int B, int C, int H, int W, 
  *          cdfo_mv_offset_head_sm100_fwd writes them (a warp's 32 pixels x gp groups are contiguous; 16-byte aligned)
  *   mv     [B, 2, H, W] fp32 (x, y) or NULL: decoded MV prior, added as offset + flow.flip(1).repeat(...) (arch:3347)
  *   wpk    73728 bytes from cdfo_dcn_tex_sm100_pack_weight (fp16); bias [64] fp32 or NULL
- *   y / out_mode / num_ctas / x_batch: as cdfo_dcn_sm100_fwd (x_batch * 16 * (H + 3) <= 65000 texture rows); fields_bstride in 8-byte elements (<= 0: dense).
+ *   y / out_mode / num_ctas / x_batch: as cdfo_dcn_sm100_fwd; fields_bstride in 8-byte elements (<= 0: dense).  The x samples are
+ *          bound as textures of at most 65000 rows (16 * (H + 3) per sample, H <= 4059); a larger x batch is split into the
+ *          fewest slices that fit, one launch per slice, with the same per-sample results.
  * Texture descriptors over x_q4t are created on first use and cached by (device, pointer, shape); they own no memory. */
 int cdfo_dcn_tex_sm100_fwd(const void *x_q4t, const void *fields, const float *mv, const void *wpk, const float *bias,
                            void *y, int B, int H, int W, int dg, int out_mode, int num_ctas, int x_batch,
@@ -249,6 +251,8 @@ int cdfo_resample_c8(const void *a, const void *b, const void *base, void *y, in
  *          separately, arch:4449);  out [B,64,H,W] fp32 = fuse(cat[long, loc]) + x + x2  arch:2246-2249
  *   tables [9 + 9 + 64 + 4096] fp32: directW1_conv taps, directH1_conv taps, K1, R (see csrc/lra.cu); beta / bh their biases
  *   fuse_w [64,128] fp32, fuse_b [64];  workspace: cdfo_lra_workspace_bytes(B, H, W) bytes;  H, W multiples of 8.
+ *   Frame bounds: W <= 1280 (rows wider than 704 run on a 2-CTA cluster), H <= 768 (the bf16 column pass; the tcgen05 one takes
+ *   H <= 384, the TF32 one H <= 384); past them CDFO_ERR_UNSUPPORTED, checked before anything is launched.
  * No score tensor is materialised (the reference writes ~3.1 kB of fp32 scores per pixel and call). */
 int cdfo_lra_fwd(const float *qv, const float *u, const float *vmax, const float *x, const float *x2, const float *tables,
                  float beta, float bh, const float *fuse_w, const float *fuse_b, float *out, void *workspace, int B, int H, int W,
@@ -257,7 +261,7 @@ int cdfo_lra_fwd(const float *qv, const float *u, const float *vmax, const float
  * half of the model's cat([fea, x_n]) (arch:4454), the input of conv_expand_fea_r; no fp32 copy of x_n exists. */
 /* Column pass operands: 0 (default) = bf16 mma.sync m16n8k16, 1 = TF32 m16n8k8 (the first-generation kernel; A/B switch). */
 int cdfo_lra_set_col_precision(int tf32);
-/* Column pass: 1 (default) = the tcgen05 kernel (csrc/lra_col_sm100.cu: score tile in tensor memory, bf16 operands; H <= 448), 0 = the
+/* Column pass: 1 (default) = the tcgen05 kernel (csrc/lra_col_sm100.cu: score tile in tensor memory, bf16 operands; H <= 384), 0 = the
  * warp-level mma.sync kernels of round 1.  A measurement / test switch. */
 int cdfo_lra_set_col_tcgen05(int on);
 /* 8x8 window pass: 1 (default) = tensor cores (bf16 hi/lo split scores, mma.sync), 0 = round 1's fp32 SIMT kernel. */

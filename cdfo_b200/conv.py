@@ -75,7 +75,7 @@ _wcache_4x4 = _lib.TensorCache()
 
 @torch.no_grad()
 def conv3x3_then_half(x8, weight, bias=None, resid8=None, up8=None, want_half=False):
-    """bilinear_x0.5(conv3x3(x8, weight) + bias) + resid8 as ONE 4x4 / stride-2 convolution on a CTA pair (cdfo_conv4x4s2_pair_sm100_fwd).
+    """bilinear_x0.5(conv3x3(x8, weight) + bias) + resid8 as ONE 4x4 / stride-2 convolution on a CTA pair (cdfo_conv4x4s2_pair_sm100_block_fwd).
     x8 [B, Cin/8, 2H, 2W, 8] bf16 -- or its parity planes [B, Cin/8, 2, 2, H, W, 8] as conv3x3(..., parity_planes=True) writes them
     (dense TMA boxes instead of stride-2 loads) -- weight [64, Cin, 3, 3] -> [B, 8, H, W, 8] bf16; resid8 at the output size.
     up8 [B, 8, H/2, W/2, 8]: its bilinear x2 is added in the epilogue; want_half: also returns bilinear_x0.5 of the result
@@ -160,7 +160,7 @@ def conv3x3(x8, weight, bias=None, act=ACT_NONE, resid8=None, out_nchw=False, pi
     pair_shape = _lib.lib().cdfo_conv3x3_pair_sm100_supported(Cout, Cin) and (parity_planes or not (Cin == 64 and Cout == 64))
     pair_ok = ks == 3 and not pixel_shuffle and not out_nchw and pair_shape
     if bias_edge is not None:
-        if not (config.conv_pair and pair_ok) or b is None or tuple(bias_edge.shape) != (9, Cout) or bias_edge.dtype != torch.float32 \
+        if not pair_ok or b is None or tuple(bias_edge.shape) != (9, Cout) or bias_edge.dtype != torch.float32 \
                 or not bias_edge.is_contiguous() or H < 2 or W < 2:
             raise _lib.CdfoError("conv3x3: bias_edge needs a CTA-pair shape, a bias and a contiguous fp32 [9, %d] table" % Cout)
         if parity_planes and (resid8 is not None or H % 2 or W % 2):
@@ -239,25 +239,12 @@ def conv_last_skip(x8, weight, bias, lr):
 
 
 @torch.no_grad()
-def resample(a, mode, b=None, base=None):
-    """c8 bf16 bilinear resampling (align_corners=False): mode 0 = x0.5 of a, 1 = x2 of a, 2 = base + x0.5(a) + x2(b),
-    3 = base + x2(b) (a is ignored)."""
-    if mode == 3:
-        B, C8, Ho, Wo, _ = base.shape
-        if tuple(b.shape) != (B, C8, Ho // 2, Wo // 2, 8) or Ho % 2 or Wo % 2 or not base.is_contiguous() or not b.is_contiguous() \
-                or base.dtype != torch.bfloat16 or b.dtype != torch.bfloat16:
-            raise _lib.CdfoError("resample: base / b shapes do not match")
-        y = torch.empty_like(base)
-        _lib.call("cdfo_resample_c8", _lib.ptr(None), _lib.ptr(b), _lib.ptr(base), _lib.ptr(y), B, C8 * 8, Ho, Wo, 3, _lib.stream_ptr(base.device))
-        return y
+def resample(a, mode):
+    """c8 bf16 bilinear resampling (align_corners=False): mode 0 = x0.5 of a (even size), 1 = x2 of a."""
     B, C8, Ha, Wa, _ = a.shape
-    Ho, Wo = (Ha // 2, Wa // 2) if mode in (0, 2) else (2 * Ha, 2 * Wa)
-    if a.dtype != torch.bfloat16 or not a.is_contiguous() or (mode != 1 and (Ha % 2 or Wa % 2)):
+    Ho, Wo = (Ha // 2, Wa // 2) if mode == 0 else (2 * Ha, 2 * Wa)
+    if a.dtype != torch.bfloat16 or not a.is_contiguous() or (mode == 0 and (Ha % 2 or Wa % 2)):
         raise _lib.CdfoError("resample: contiguous bf16 c8 input with even size expected")
-    if mode == 2 and (tuple(base.shape) != (B, C8, Ho, Wo, 8) or tuple(b.shape) != (B, C8, Ho // 2, Wo // 2, 8)
-                      or not base.is_contiguous() or not b.is_contiguous()):
-        raise _lib.CdfoError("resample: base / b shapes do not match")
     y = torch.empty((B, C8, Ho, Wo, 8), dtype=torch.bfloat16, device=a.device)
-    _lib.call("cdfo_resample_c8", _lib.ptr(a), _lib.ptr(b), _lib.ptr(base), _lib.ptr(y), B, C8 * 8, Ho, Wo, int(mode),
-              _lib.stream_ptr(a.device))
+    _lib.call("cdfo_resample_c8", _lib.ptr(a), _lib.ptr(y), B, C8 * 8, Ho, Wo, int(mode), _lib.stream_ptr(a.device))
     return y

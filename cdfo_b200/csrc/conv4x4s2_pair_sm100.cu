@@ -355,41 +355,26 @@ extern "C" int cdfo_conv4x4s2_pair_sm100_pack_weight(const float *w3, void *wpk,
   return check_launch("cdfo_conv4x4s2_pair_sm100_pack_weight");
 }
 
-extern "C" int cdfo_conv4x4s2_pair_sm100_planes_fwd(const void *x, const void *wpk, const float *bias, const void *resid_c8, void *y_c8,
-                                                    int B, int Cin, int H_in, int W_in, int x_planes, void *stream);
-extern "C" int cdfo_conv4x4s2_pair_sm100_block_fwd(const void *x, const void *wpk, const float *bias, const void *resid_c8, const void *up_c8,
-                                                   void *y_c8, void *half_c8, int B, int Cin, int H_in, int W_in, int x_planes, void *stream);
-
-extern "C" int cdfo_conv4x4s2_pair_sm100_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, void *y_c8, int B,
-                                             int Cin, int H_in, int W_in, void *stream) {
-  return cdfo_conv4x4s2_pair_sm100_planes_fwd(x_c8, wpk, bias, resid_c8, y_c8, B, Cin, H_in, W_in, 0, stream);
-}
-
-extern "C" int cdfo_conv4x4s2_pair_sm100_planes_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, void *y_c8,
-                                                    int B, int Cin, int H_in, int W_in, int x_planes, void *stream) {
-  return cdfo_conv4x4s2_pair_sm100_block_fwd(x_c8, wpk, bias, resid_c8, nullptr, y_c8, nullptr, B, Cin, H_in, W_in, x_planes, stream);
-}
-
 extern "C" int cdfo_conv4x4s2_pair_sm100_block_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, const void *up_c8,
                                                    void *y_c8, void *half_c8, int B, int Cin, int H_in, int W_in, int x_planes, void *stream) {
-  CDFO_REQUIRE(x_c8 && wpk && y_c8, CDFO_ERR_NULL, "cdfo_conv4x4s2_pair_sm100_fwd: NULL pointer");
+  CDFO_REQUIRE(x_c8 && wpk && y_c8, CDFO_ERR_NULL, "cdfo_conv4x4s2_pair_sm100_block_fwd: NULL pointer");
   CDFO_REQUIRE((!up_c8 && !half_c8) || (H_in % 4 == 0 && W_in % 4 == 0), CDFO_ERR_SHAPE,
                "cdfo_conv4x4s2_pair_sm100_block_fwd: up_c8 / half_c8 need an even output size (input %d x %d)", H_in, W_in);
   CDFO_REQUIRE(((uintptr_t)up_c8 & 15) == 0 && ((uintptr_t)half_c8 & 15) == 0, CDFO_ERR_SHAPE,
                "cdfo_conv4x4s2_pair_sm100_block_fwd: pointers must be 16-byte aligned");
-  CDFO_REQUIRE(x_planes == 0 || x_planes == 1, CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_planes_fwd: x_planes %d", x_planes);
+  CDFO_REQUIRE(x_planes == 0 || x_planes == 1, CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_block_fwd: x_planes %d", x_planes);
   CDFO_REQUIRE(B > 0 && H_in > 0 && W_in > 0 && H_in % 2 == 0 && W_in % 2 == 0, CDFO_ERR_SHAPE,
-               "cdfo_conv4x4s2_pair_sm100_fwd: the input size must be even (got %d x %d)", H_in, W_in);
-  CDFO_REQUIRE(cdfo_conv4x4s2_pair_sm100_supported(64, Cin), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_fwd: unsupported input channels %d", Cin);
+               "cdfo_conv4x4s2_pair_sm100_block_fwd: the input size must be even (got %d x %d)", H_in, W_in);
+  CDFO_REQUIRE(cdfo_conv4x4s2_pair_sm100_supported(64, Cin), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_block_fwd: unsupported input channels %d", Cin);
   CDFO_REQUIRE(((uintptr_t)x_c8 & 15) == 0 && ((uintptr_t)wpk & 15) == 0 && ((uintptr_t)y_c8 & 15) == 0 && ((uintptr_t)resid_c8 & 15) == 0,
-               CDFO_ERR_SHAPE, "cdfo_conv4x4s2_pair_sm100_fwd: pointers must be 16-byte aligned");
+               CDFO_ERR_SHAPE, "cdfo_conv4x4s2_pair_sm100_block_fwd: pointers must be 16-byte aligned");
   c4::EncodeTiledFn enc = c4::encode_tiled_fn();
-  CDFO_REQUIRE(enc, CDFO_ERR_CUDA, "cdfo_conv4x4s2_pair_sm100_fwd: cuTensorMapEncodeTiled not available from the driver");
+  CDFO_REQUIRE(enc, CDFO_ERR_CUDA, "cdfo_conv4x4s2_pair_sm100_block_fwd: cuTensorMapEncodeTiled not available from the driver");
   CUtensorMap xm, wm;
   if (x_planes) {
     // [B * Cin/8][4 planes][H][W][8]: a box of 4 channel chunks starts at a multiple of 4 and never crosses a sample
     const cuuint64_t Ho = H_in / 2, Wo = W_in / 2;
-    CDFO_REQUIRE((long long)B * (Cin / 8) < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_planes_fwd: too many chunks");
+    CDFO_REQUIRE((long long)B * (Cin / 8) < (1ll << 31), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_block_fwd: too many chunks");
     // the pixel and channel axes are merged (a window row of 9 pixels = 72 contiguous elements): 17 x 4 requests of 144 bytes per
     // box instead of 9 x 17 x 4 of 16 bytes
     const cuuint64_t gdim[5] = {Wo * 8, Ho, 4, (cuuint64_t)B * (Cin / 8), 1};
@@ -424,7 +409,7 @@ extern "C" int cdfo_conv4x4s2_pair_sm100_block_fwd(const void *x_c8, const void 
   p.B = B; p.Cin = Cin; p.H = H_in / 2; p.W = W_in / 2; p.x_planes = x_planes;
   p.tiles_x = ceil_div(p.W, c4::kTileW); p.tiles_y = ceil_div(p.H, c4::kTileH);
   const long long mt = (long long)B * p.tiles_x * p.tiles_y;
-  CDFO_REQUIRE(mt < (1ll << 30), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_fwd: too many tiles");
+  CDFO_REQUIRE(mt < (1ll << 30), CDFO_ERR_UNSUPPORTED, "cdfo_conv4x4s2_pair_sm100_block_fwd: too many tiles");
   p.m_tiles = (int)mt;
   static bool attr_done = false;
   static int max_pairs = kNumSMs / 2;
@@ -444,5 +429,5 @@ extern "C" int cdfo_conv4x4s2_pair_sm100_block_fwd(const void *x_c8, const void 
   int pairs = (p.m_tiles + 1) / 2;
   if (pairs > max_pairs) pairs = max_pairs;
   c4::conv4x4s2_pair_sm100_kernel<<<pairs * 2, c4::kThreads, c4::kSmem, (cudaStream_t)stream>>>(xm, wm, p);
-  return check_launch("cdfo_conv4x4s2_pair_sm100_fwd");
+  return check_launch("cdfo_conv4x4s2_pair_sm100_block_fwd");
 }

@@ -416,56 +416,32 @@ def _block_weights(blk):
 
 @torch.no_grad()
 def cross_scale_block(blk, x8, x8_half=None, want_half=False):
-    """Block_.forward, arch:401-406, on c8 bf16.  Bilinear x0.5 / x2 commute with the 1x1 convs (per-pixel linear maps whose
-    bias passes through weights that sum to 1), so every 1x1 runs at the lower of its two resolutions, and the 1x1 that
-    follows a body is composed into the body's second 3x3:
+    """Block_.forward, arch:401-406, on c8 bf16 [B, 8, H, W, 8] with H and W even and >= 4.  Bilinear x0.5 / x2 commute with the 1x1
+    convs (per-pixel linear maps whose bias passes through weights that sum to 1), so each 1x1 of down / up is composed into the body's
+    first 3x3 (border-class bias table) and the 1x1 that follows a body into the body's second 3x3:
         x + body(x)                         two convs at 1x (residual add in the epilogue)
-        up(body(down(x)))                   x0.5 -> 1x1 -> conv -> conv o up-1x1 at 1/2x, then x2
-        down(body(up(x)))                   1x1 at 1x -> x2 -> conv -> conv o down-1x1 at 2x, then x0.5
-    and the three branches are summed in the epilogue of the last convolution (config.trunk_fused_resample; a resampling kernel
-    otherwise).  x8_half: bilinear x0.5 of x8 if the producer of x8 already wrote it; want_half: return (out, x0.5 of out)."""
+        up(body(down(x)))                   x0.5 -> conv o down-1x1 -> conv o up-1x1 at 1/2x, then x2
+        down(body(up(x)))                   conv o up-1x1 at 2x, its input the bilinear x2 of x built in the kernel's producer and its output
+                                            the four parity planes -> conv o down-1x1 and x0.5 as one 4x4 / stride-2 convolution at 1x
+    The last kernel also adds the other two branches in its epilogue.  x8_half: bilinear x0.5 of x8 if the producer of x8 already
+    wrote it; want_half: return (out, x0.5 of out), the x0.5 taken in the same epilogue."""
+    H, W = x8.shape[2:4]
+    if H % 2 or W % 2 or H < 4 or W < 4:
+        raise _lib.CdfoError("cross_scale_block: H and W must be even and >= 4 (got %d x %d)" % (H, W))
     b0, b2 = blk.body._modules["0"], blk.body._modules["2"]
-    dn, up = blk.down._modules["0"], blk.up._modules["0"]
     wts = _block_weights(blk)
+    wd0, bd0, ed0 = wts["body0_dn"]
+    wu0, bu0, eu0 = wts["body0_up"]
     y = conv.conv3x3(conv.conv3x3(x8, b0.weight, b0.bias, conv.ACT_LRELU), b2.weight, b2.bias, conv.ACT_NONE, resid8=x8)
-    fused = config.trunk_fused_resample and config.conv_fold_half and x8.size(2) % 2 == 0 and x8.size(3) % 2 == 0
     xh = x8_half if x8_half is not None else conv.resample(x8, 0)
-    compose = config.trunk_compose_1x1 and config.conv_pair and min(xh.shape[2:4]) >= 2
-    if compose:
-        # the down / up 1x1 convolutions live inside body.0's weights (border-aware bias): no 1x1 launches, body.0 reads the resampled x
-        wd0, bd0, ed0 = wts["body0_dn"]
-        wu0, bu0, eu0 = wts["body0_up"]
-        cu = conv.conv3x3(conv.conv3x3(xh, wd0, bd0, conv.ACT_LRELU, bias_edge=ed0), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
-        # config.trunk_fused_upsample: body.0 at 2x evaluates the bilinear x2 of x8 itself (no 2x input tensor in HBM)
-        xu = None if config.trunk_fused_upsample and config.conv_fold_half else conv.resample(x8, 1)
-    else:
-        xd = conv.conv3x3(xh, dn.weight, dn.bias, conv.ACT_NONE)            # 1x1
-        cu = conv.conv3x3(conv.conv3x3(xd, b0.weight, b0.bias, conv.ACT_LRELU), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
-        xu = conv.resample(conv.conv3x3(x8, up.weight, up.bias, conv.ACT_NONE), 1)               # 1x1
-        wu0, bu0, eu0 = b0.weight, b0.bias, None
-    if config.conv_fold_half:
-        # the 2x-resolution intermediate lives as its four parity planes: the stride-2 taps of the folded convolution are dense boxes
-        planes = config.conv_parity_planes and config.conv_pair
-        if xu is None:
-            t2 = conv.conv3x3_up2(x8, wu0, bu0, conv.ACT_LRELU, parity_planes=planes, bias_edge=eu0)
-        else:
-            t2 = conv.conv3x3(xu, wu0, bu0, conv.ACT_LRELU, parity_planes=planes, bias_edge=eu0)
-        # bilinear x0.5 of a 3x3 convolution = one 4x4 / stride-2 convolution: evaluated at 1x, the branch sum starts in its epilogue
-        if fused:
-            # ... and ends there: + bilinear x2 of the half-resolution branch, and the x0.5 of the sum for the next block's down branch
-            return conv.conv3x3_then_half(t2, wts["dn_body2"][0], wts["dn_body2"][1], resid8=y, up8=cu, want_half=want_half)
-        yb = conv.conv3x3_then_half(t2, wts["dn_body2"][0], wts["dn_body2"][1], resid8=y)
-        out = conv.resample(None, 3, b=cu, base=yb)
-    else:
-        t2 = conv.conv3x3(xu, wu0, bu0, conv.ACT_LRELU, bias_edge=eu0)
-        b3 = conv.conv3x3(t2, wts["dn_body2"][0], wts["dn_body2"][1], conv.ACT_NONE)
-        out = conv.resample(b3, 2, b=cu, base=y)
-    return (out, None) if want_half else out
+    cu = conv.conv3x3(conv.conv3x3(xh, wd0, bd0, conv.ACT_LRELU, bias_edge=ed0), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
+    t2 = conv.conv3x3_up2(x8, wu0, bu0, conv.ACT_LRELU, parity_planes=True, bias_edge=eu0)
+    return conv.conv3x3_then_half(t2, wts["dn_body2"][0], wts["dn_body2"][1], resid8=y, up8=cu, want_half=want_half)
 
 
 @torch.no_grad()
 def recon_trunk(trunk, x8):
-    """SCNet_(7 x SCGroup_(3 x Block_)), arch:430-480, c8 bf16 in and out."""
+    """SCNet_(7 x SCGroup_(3 x Block_)), arch:430-480, c8 bf16 in and out; H and W even and >= 4 (cross_scale_block)."""
     y = x8
     for grp in trunk.body._modules.values():
         r, r_half = y, None

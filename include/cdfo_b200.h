@@ -239,10 +239,9 @@ int cdfo_channel_gate_fwd(const float *partial_sums, int parts, const float *w1,
 int cdfo_pack_c8_scaled(const float *x_nchw, const float *scale, void *x_c8, int B, int C, int H, int W, void *stream);
 int cdfo_unpack_c8_add(const void *x_c8, const float *add_nchw, int add_batch, float *y_nchw, int B, int C, int H, int W,
                        void *stream);
-/* ---- bilinear x0.5 / x2 (align_corners=False, arch/SIDECVSR_our.py:324-333) on c8 bf16, and the three-scale sum of the
- * trunk's cross-scale block (arch:401-406).  mode 0: y [B,C/8,Ho,Wo,8] = x0.5(a [.,2Ho,2Wo,.]); mode 1: y = x2(a [.,Ho/2,Wo/2,.]);
- * mode 2: y = base + x0.5(a) + x2(b). */
-int cdfo_resample_c8(const void *a, const void *b, const void *base, void *y, int B, int C, int Ho, int Wo, int mode, void *stream);
+/* ---- bilinear x0.5 / x2 (align_corners=False, arch/SIDECVSR_our.py:324-333) on c8 bf16.  mode 0: y [B,C/8,Ho,Wo,8] = x0.5(a [.,2Ho,2Wo,.]);
+ * mode 1: y = x2(a [.,Ho/2,Wo/2,.]) (Ho, Wo even). */
+int cdfo_resample_c8(const void *a, void *y, int B, int C, int Ho, int Wo, int mode, void *stream);
 /* ---- A8: LLongRangAttention.forward (arch/SIDECVSR_our.py:2179-2249) after its 1x1 input_conv and the pooled mask logits ----
  *   qv     [B,128,H,W] fp32 = input_conv(x) (q = first 64 channels, v = last 64)          arch:2206,2211
  *   u      [B,64,H,W]  fp32 uniform noise of gumbel_softmax (torch.rand_like, arch:2169)
@@ -304,7 +303,7 @@ int cdfo_conv3x3_pair_sm100_pack_weight(const float *w, void *wpk, int Cout, int
 int cdfo_conv3x3_pair_sm100_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, void *y_c8, int B, int Cin,
                                 int Cout, int H, int W, int act, void *stream);
 /* Same, with y_planes = 1 storing the output as its four parity planes [B,Cout/8,2 (row parity),2 (column parity),H/2,W/2,8]
- * (H, W even; pixel (h, w) -> plane (h & 1, w & 1) at (h / 2, w / 2)): the input layout of cdfo_conv4x4s2_pair_sm100_planes_fwd;
+ * (H, W even; pixel (h, w) -> plane (h & 1, w & 1) at (h / 2, w / 2)): the x_planes = 1 input layout of cdfo_conv4x4s2_pair_sm100_block_fwd;
  * y_planes = 2: y is NCHW fp32 [B,Cout,H,W]. */
 int cdfo_conv3x3_pair_sm100_planes_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, void *y, int B,
                                        int Cin, int Cout, int H, int W, int act, int y_planes, void *stream);
@@ -321,20 +320,16 @@ int cdfo_conv3x3_pair_sm100_up2_fwd(const void *x8_1x, const void *wpk, const fl
 /* ---- "3x3 convolution at 2H x 2W followed by bilinear x0.5" as ONE 4x4 / stride-2 convolution on a CTA pair
  * (csrc/conv4x4s2_pair_sm100.cu): the down(body(up(x))) branch of Block_.forward, arch/SIDECVSR_our.py:401-406 with Interpolate(0.5)
  * :324-333.  w3 [64,Cin,3,3] fp32 is the 3x3 weight (pack_weight folds the 2x2 mean into a 4x4 kernel);
- * x_c8 [B,Cin/8,H_in,W_in,8] bf16 (H_in, W_in even) -> y_c8 [B,8,H_in/2,W_in/2,8] bf16 = conv + bias + resid_c8. */
-int cdfo_conv4x4s2_pair_sm100_supported(int Cout, int Cin);
-size_t cdfo_conv4x4s2_pair_sm100_weight_bytes(int Cin);
-int cdfo_conv4x4s2_pair_sm100_pack_weight(const float *w3, void *wpk, int Cin, void *stream);
-int cdfo_conv4x4s2_pair_sm100_fwd(const void *x_c8, const void *wpk, const float *bias, const void *resid_c8, void *y_c8, int B, int Cin,
-                                  int H_in, int W_in, void *stream);
-/* Same, with x_planes = 1 reading x as parity planes [B,Cin/8,2,2,H_in/2,W_in/2,8]: every stride-2 phase window is then a dense
- * TMA box (the plain c8 input is loaded with elementStrides = 2, one L2 request per 16-byte pixel chunk). */
-int cdfo_conv4x4s2_pair_sm100_planes_fwd(const void *x, const void *wpk, const float *bias, const void *resid_c8, void *y_c8, int B,
-                                         int Cin, int H_in, int W_in, int x_planes, void *stream);
-/* Same, closing a whole cross-scale block (Block_.forward, arch/SIDECVSR_our.py:401-406) in the epilogue:
+ * x [B,Cin/8,H_in,W_in,8] bf16 (H_in, W_in even) -> y_c8 [B,8,H_in/2,W_in/2,8] bf16 = conv + bias + resid_c8.  x_planes = 1 reads x as
+ * parity planes [B,Cin/8,2,2,H_in/2,W_in/2,8]: every stride-2 phase window is then a dense TMA box (the plain c8 input, x_planes = 0, is
+ * loaded with elementStrides = 2, one L2 request per 16-byte pixel chunk).  The epilogue can close a whole cross-scale block
+ * (Block_.forward, arch/SIDECVSR_our.py:401-406):
  *   y = conv + bias + resid_c8 + bilinear_x2(up_c8)        up_c8 [B,8,H_in/4,W_in/4,8] bf16 or NULL: the up(body(down(x))) branch
  *   half_c8 = bilinear_x0.5(y) from the fp32 values        [B,8,H_in/4,W_in/4,8] bf16 or NULL: the next block's down(x) input
  * (no separate resampling passes over HBM; H_in, W_in multiples of 4 when either is given). */
+int cdfo_conv4x4s2_pair_sm100_supported(int Cout, int Cin);
+size_t cdfo_conv4x4s2_pair_sm100_weight_bytes(int Cin);
+int cdfo_conv4x4s2_pair_sm100_pack_weight(const float *w3, void *wpk, int Cin, void *stream);
 int cdfo_conv4x4s2_pair_sm100_block_fwd(const void *x, const void *wpk, const float *bias, const void *resid_c8, const void *up_c8,
                                         void *y_c8, void *half_c8, int B, int Cin, int H_in, int W_in, int x_planes, void *stream);
 /* ---- frame I/O of the evaluation loop (SURVEY 8f rank 3) ----

@@ -10,7 +10,7 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("H,W", [(8, 8), (24, 40), (34, 50)])
-def test_resample_c8_vs_interpolate(cuda_dev, H, W):
+def test_resample_c8_half_and_double_vs_interpolate(cuda_dev, H, W):
     from cdfo_b200 import conv
     g = torch.Generator().manual_seed(H * W)
     x = torch.randn(2, 64, H, W, generator=g).to(torch.bfloat16).float().to(cuda_dev)
@@ -21,37 +21,27 @@ def test_resample_c8_vs_interpolate(cuda_dev, H, W):
     dn = conv.from_c8(conv.resample(x8, 0))
     ref_dn = F.interpolate(x, scale_factor=0.5, mode="bilinear", align_corners=False)
     assert (dn - ref_dn).abs().max().item() <= 2 ** -8 * ref_dn.abs().max().item()
-    big = torch.randn(2, 64, 2 * H, 2 * W, generator=g).to(torch.bfloat16).float().to(cuda_dev)
-    small = torch.randn(2, 64, H // 2, W // 2, generator=g).to(torch.bfloat16).float().to(cuda_dev)
-    got = conv.from_c8(conv.resample(conv.to_c8(big), 2, b=conv.to_c8(small), base=x8))
-    ref = x + F.interpolate(big, scale_factor=0.5, mode="bilinear", align_corners=False) + \
-        F.interpolate(small, scale_factor=2.0, mode="bilinear", align_corners=False)
-    assert (got - ref).abs().max().item() <= 2 ** -8 * ref.abs().max().item()
 
 
-@pytest.mark.parametrize("fused,compose", [(True, True), (True, False), (False, False)])
-def test_trunk_vs_oracle(cuda_dev, fused, compose):
-    """SCNet_ (21 cross-scale blocks) on c8 bf16 with composed 1x1 convolutions vs the fp32 oracle (arch:378-480), with the block sums in
-    the folded convolution's epilogue and the down / up 1x1 convolutions composed into body.0 (default), and with round 1's separate kernels.  Observed on the B200: 7.2e-3 / 7.4e-3 of max|ref|
-    (21 blocks of bf16 activations); the bound is 1e-2."""
-    from cdfo_b200 import config, conv, hotpath
+# the model's 24 x 40 test size; two samples at 16 x 24; 18 x 30, whose half-size images (9 x 15) are odd, with ragged tiles at every scale
+@pytest.mark.parametrize("B,H,W", [(1, 24, 40), (2, 16, 24), (1, 18, 30)])
+def test_trunk_vs_oracle(cuda_dev, B, H, W):
+    """SCNet_ (21 cross-scale blocks) on c8 bf16 with composed 1x1 convolutions and the block sums in the folded convolution's epilogue
+    vs the fp32 oracle (arch:378-480).  Observed on the B200 at 1 x 24 x 40: 7.2e-3 of max|ref| (21 blocks of bf16 activations); the
+    bound is 1e-2."""
+    from cdfo_b200 import conv, hotpath
     from cdfo_b200.model import CVSR_V8
     sd = G.seeded_weights("O1")
     m = CVSR_V8()
     m.load_state_dict(sd, strict=True)
     m = m.to(cuda_dev).eval()
     g = torch.Generator().manual_seed(5)
-    x = torch.randn(1, 64, 24, 40, generator=g)
+    x = torch.randn(B, 64, H, W, generator=g)
     with torch.no_grad():
         ref = torch_ref.trunk(sd, x)
-    keep = config.trunk_fused_resample, config.trunk_compose_1x1
-    try:
-        config.trunk_fused_resample, config.trunk_compose_1x1 = fused, compose
-        got = conv.from_c8(hotpath.recon_trunk(m.recon_trunk, conv.to_c8(x.to(cuda_dev)))).cpu()
-    finally:
-        config.trunk_fused_resample, config.trunk_compose_1x1 = keep
+    got = conv.from_c8(hotpath.recon_trunk(m.recon_trunk, conv.to_c8(x.to(cuda_dev)))).cpu()
     err = (got - ref).abs().max().item()
-    print("trunk (fused resampling %s, composed 1x1 %s) max err %.3g (max|ref| %.3g)" % (fused, compose, err, ref.abs().max().item()))
+    print("trunk %d x %d x %d max err %.3g (max|ref| %.3g)" % (B, H, W, err, ref.abs().max().item()))
     assert err <= 1e-2 * ref.abs().max().item()
 
 

@@ -1,6 +1,7 @@
 """The index arithmetic of the UP2 A-operand builder (csrc/conv3x3_pair_sm100.cu) restated in numpy: a tile's 18 x 10 halo of
 bilinear_x2(x), rebuilt from the edge-clamped 10 x 6 source window, equals F.interpolate's values with zero padding outside the 2x frame.
-Inputs are multiples of 16 below 2^12, so every blend is exact and the comparison is exact too.  Argument checks of the C entry point."""
+Inputs are multiples of 16 below 2^12, so every blend is exact and the comparison is exact too.  Argument checks of the C entry point
+and of hotpath.cross_scale_block."""
 import ctypes
 
 import numpy as np
@@ -66,3 +67,14 @@ def test_up2_entry_point_rejects_bad_arguments(cdfo_so):
     assert b"even" in lib.cdfo_last_error()
     assert fn(buf, buf, None, None, buf, 1, 64, 256, 16, 16, 2, 2, None) != 0
     assert b"y_planes" in lib.cdfo_last_error()
+
+
+@pytest.mark.parametrize("H,W", [(15, 16), (16, 9), (2, 16), (16, 2), (3, 3)])
+def test_cross_scale_block_rejects_odd_or_small_frames(H, W):
+    """The block's kernels need even sides (x0.5, parity planes) and a half-size image of at least 2 x 2 (border-class bias): other sizes
+    are refused with a message naming the bound, before any CUDA call (this runs without a device)."""
+    from cdfo_b200 import _lib, hotpath
+    from cdfo_b200.model import _CrossScaleBlock
+    x8 = torch.zeros(1, 8, H, W, 8, dtype=torch.bfloat16)
+    with pytest.raises(_lib.CdfoError, match=r"even and >= 4 \(got %d x %d\)" % (H, W)):
+        hotpath.cross_scale_block(_CrossScaleBlock(), x8, want_half=True)

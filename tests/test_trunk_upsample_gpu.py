@@ -32,21 +32,40 @@ def test_conv3x3_up2_equals_resample_then_conv(cuda_dev, B, H, W):
     assert torch.equal(conv.conv3x3_up2(x8, w, None, conv.ACT_NONE), ref)
 
 
-def test_recon_trunk_fused_upsample_is_bit_exact(cuda_dev):
+def _block_with_resample(blk, x8, x8_half, want_half):
+    """hotpath.cross_scale_block with body.0 at 2x reading the output of the x2 resample kernel instead of building it in its producer."""
+    from cdfo_b200 import conv, hotpath
+    b0, b2 = blk.body._modules["0"], blk.body._modules["2"]
+    wts = hotpath._block_weights(blk)
+    wd0, bd0, ed0 = wts["body0_dn"]
+    wu0, bu0, eu0 = wts["body0_up"]
+    y = conv.conv3x3(conv.conv3x3(x8, b0.weight, b0.bias, conv.ACT_LRELU), b2.weight, b2.bias, conv.ACT_NONE, resid8=x8)
+    xh = x8_half if x8_half is not None else conv.resample(x8, 0)
+    cu = conv.conv3x3(conv.conv3x3(xh, wd0, bd0, conv.ACT_LRELU, bias_edge=ed0), wts["up_body2"][0], wts["up_body2"][1], conv.ACT_NONE)
+    t2 = conv.conv3x3(conv.resample(x8, 1), wu0, bu0, conv.ACT_LRELU, parity_planes=True, bias_edge=eu0)
+    return conv.conv3x3_then_half(t2, wts["dn_body2"][0], wts["dn_body2"][1], resid8=y, up8=cu, want_half=want_half)
+
+
+def test_recon_trunk_upsample_in_body0_is_bit_exact(cuda_dev):
     """The whole trunk (21 cross-scale blocks) at the c3 size with the upsample inside body.0 and with the resample kernel."""
-    from cdfo_b200 import config, conv, hotpath
+    from cdfo_b200 import conv, hotpath
     from cdfo_b200.model import CVSR_V8
     m = CVSR_V8()
     m.load_state_dict(G.seeded_weights("O1"), strict=True)
     m = m.to(cuda_dev).eval()
     g = torch.Generator().manual_seed(7)
     x8 = conv.to_c8(torch.randn(1, 64, 272, 480, generator=g).to(cuda_dev))
-    keep = config.trunk_fused_upsample
-    try:
-        config.trunk_fused_upsample = False
-        ref = hotpath.recon_trunk(m.recon_trunk, x8)
-        config.trunk_fused_upsample = True
-        got = hotpath.recon_trunk(m.recon_trunk, x8)
-    finally:
-        config.trunk_fused_upsample = keep
+    with torch.no_grad():
+        ref = x8
+        for grp in m.recon_trunk.body._modules.values():               # hotpath.recon_trunk's loop
+            r, r_half = ref, None
+            blocks = list(grp.body._modules.values())
+            for k, blk in enumerate(blocks):
+                if k + 1 < len(blocks):
+                    r, r_half = _block_with_resample(blk, r, r_half, want_half=True)
+                else:
+                    r = _block_with_resample(blk, r, r_half, want_half=False)
+            ref = conv.conv3x3(r, grp.conv.weight, grp.conv.bias, conv.ACT_NONE, resid8=ref)
+        ref = ref + x8
+    got = hotpath.recon_trunk(m.recon_trunk, x8)
     assert torch.equal(got, ref)

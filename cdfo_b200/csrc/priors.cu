@@ -74,6 +74,40 @@ __global__ void mv_slot_kernel(float *__restrict__ flows, int B, int slot_elems,
   }
 }
 
+// A2 per sample: one thread per (pixel, sample) holds both flow components of the 7 frames in registers and applies the six
+// conditional slot copies of modify_mv_for_end_frames in the reference's statement order (test_LD_37.py:209-234), with the
+// sample's own (i, max_idx) from the device table i_max [B, 2].  Only the frame slots a condition rewrote are stored.
+__global__ void mv_end_fix_batched_kernel(float *__restrict__ flows, int HW, const int *__restrict__ i_max) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+  if (p >= HW) return;
+  const int i = __ldg(i_max + 2 * b), m = __ldg(i_max + 2 * b + 1);
+  const bool lo = i >= 0 && i <= 2, hi = i >= m - 3 && i <= m - 1;
+  if (!lo && !hi) return;
+  const size_t slot = 2 * (size_t)HW;
+  float *base = flows + (size_t)b * 7 * slot + p;
+#pragma unroll
+  for (int c = 0; c < 2; ++c) {
+    float *f = base + (size_t)c * HW;
+    float v[7];
+#pragma unroll
+    for (int t = 0; t < 7; ++t) v[t] = f[t * slot];
+    if (i == 0) { v[0] = 0.f; v[1] = 0.f; v[2] = 0.f; }
+    if (i == 1) { v[0] = v[2]; v[1] = v[2]; }
+    if (i == 2) { v[0] = v[1]; }
+    if (i == m - 1) { v[4] = 0.f; v[5] = 0.f; v[6] = 0.f; }
+    if (i == m - 2) { v[5] = v[4]; v[6] = v[4]; }
+    if (i == m - 3) { v[6] = v[5]; }
+    if (lo) {
+#pragma unroll
+      for (int t = 0; t < 3; ++t) f[t * slot] = v[t];
+    }
+    if (hi) {
+#pragma unroll
+      for (int t = 4; t < 7; ++t) f[t * slot] = v[t];
+    }
+  }
+}
+
 // ---------------------------------------------------------------- A3
 constexpr int kWarpCh = 8;  // channels per thread
 
@@ -222,6 +256,15 @@ extern "C" int cdfo_mv_end_fix(float *flows, int B, int H, int W, int i, int max
   if (i == max_idx - 2) { op(5, 4); op(6, 4); }
   if (i == max_idx - 3) { op(6, 5); }
   return check_launch("cdfo_mv_end_fix");
+}
+
+extern "C" int cdfo_mv_end_fix_batched(float *flows, int B, int H, int W, const int *i_max, void *stream) {
+  CDFO_REQUIRE(flows && i_max, CDFO_ERR_NULL, "cdfo_mv_end_fix_batched: NULL pointer");
+  CDFO_REQUIRE(B > 0 && B <= 65535 && H > 0 && W > 0 && (long long)H * W <= INT_MAX / 2, CDFO_ERR_SHAPE,
+               "cdfo_mv_end_fix_batched: bad shape B=%d H=%d W=%d", B, H, W);
+  const int HW = H * W;
+  mv_end_fix_batched_kernel<<<dim3(ceil_div(HW, 256), B), 256, 0, (cudaStream_t)stream>>>(flows, HW, i_max);
+  return check_launch("cdfo_mv_end_fix_batched");
 }
 
 extern "C" int cdfo_flow_warp_fwd(const float *x, const float *flow, float *y, int B, int C, int H, int W,

@@ -312,6 +312,14 @@ class FeatureRing:
     def window(self):
         return self.buf[self.head:self.head + self.N]
 
+    def load(self, b, frames):
+        """Window positions 1 .. len(frames) of batch sample b (both copies) := frames, each [C, H, W]: the features a sample needs
+        before the next push to hold a new window (frame driver admission; position 0 is pushed out by that step)."""
+        for p, f in enumerate(frames, 1):
+            t = (self.head + p) % self.N
+            self.buf[t, b].copy_(f)
+            self.buf[t + self.N, b].copy_(f)
+
     def handle(self):
         """What forward() returns as L1_fea in ring mode: a view of the window (FRAME-major [N*B, C, H, W]; equal to the
         reference's tensor for B = 1) tagged with the ring, valid until the next step."""
@@ -376,6 +384,21 @@ class CVSR_V8(nn.Module):
             with torch.autocast("cuda", dtype=dt):
                 return self.recon_trunk(x.contiguous(memory_format=torch.channels_last)).float()
         return self.recon_trunk(x)
+
+    @torch.no_grad()
+    def load_window_features(self, l1, b, x, pms, order):
+        """Starts a new window in batch sample b of a running sequence of steps: computes the L1 features of the distinct frames
+        x, pms [n, 1, H, W] and writes feature order[p] to window position p + 1 (p = 0..5) of `l1`, the L1_fea the previous step
+        returned (a FeatureRing handle or the batch-major [B*N, C, H, W] tensor).  The next step's push of its new frame then leaves
+        sample b with the features of the whole new window, as if it had started with it."""
+        f = self._features(x, pms)
+        ring = getattr(l1, "_cdfo_ring", None)
+        if ring is not None:
+            ring[0].load(b, [f[k] for k in order])
+            return
+        win = l1.view(-1, 2 * self.center + 1, *l1.shape[1:])[b]
+        for p, k in enumerate(order, 1):
+            win[p].copy_(f[k])
 
     @torch.no_grad()
     def forward(self, x, mvs0, mvs1, pms, rms, ufs, pre_L1_fea=None, noise=None):

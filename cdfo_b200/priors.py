@@ -60,6 +60,22 @@ def modify_mv_for_end_frames(i: int, mvs: torch.Tensor, max_idx: int) -> torch.T
 
 
 @torch.no_grad()
+def modify_mv_for_end_frames_batched(mvs: torch.Tensor, i_max: torch.Tensor) -> torch.Tensor:
+    """The same fix-up with its own (i, max_idx) per sample: i_max is a CUDA int32 [B, 2] table on the device of mvs (frame
+    driver slots sit at different frames of different sequences).  One launch, in place on mvs [B, 7, 2, H, W]; returns mvs."""
+    _lib.require_cuda(mvs, i_max)
+    if mvs.dim() != 5 or mvs.size(1) != 7 or mvs.size(2) != 2 or mvs.dtype != torch.float32:
+        raise ValueError("mvs must be fp32 [B, 7, 2, H, W]")
+    if not mvs.is_contiguous():
+        raise RuntimeError("mvs has to be contiguous")
+    B, _, _, H, W = mvs.shape
+    if i_max.dtype != torch.int32 or tuple(i_max.shape) != (B, 2) or not i_max.is_contiguous() or i_max.device != mvs.device:
+        raise ValueError("i_max must be a contiguous int32 [B, 2] tensor on the device of mvs")
+    _lib.call("cdfo_mv_end_fix_batched", _lib.ptr(mvs), B, H, W, _lib.ptr(i_max), _lib.stream_ptr(mvs.device))
+    return mvs
+
+
+@torch.no_grad()
 def flow_warp(x, flow, interp_mode="bilinear", padding_mode="zeros", align_corners=True, return_index=False):
     """x [B,C,H,W] fp32, flow [B,H,W,2] (the reference's argument layout, last dim = (x, y))."""
     if interp_mode != "bilinear" or padding_mode != "zeros" or not align_corners:

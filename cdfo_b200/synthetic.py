@@ -114,14 +114,25 @@ class SyntheticSequences:
     """Lazy list of `n` synthetic coded sequences in the reference's on-disk data contract (driver.Sequence: uint8 LR / partition /
     unfiltered planes, integer residual maps, int8 MV fields [T, h, W, 3], uint8 ground truth at x4), each a pure function of its
     sequence id -- a rank generates only the sequences it owns, and every sharding sees identical data (BASELINE.json configs[3]:
-    64 independent 1080p x4 sequences)."""
+    64 independent 1080p x4 sequences).  `frames`, `h`, `w` are one value for every sequence or one per sequence (a job of mixed sizes
+    and lengths, tools/bench_job.py)."""
 
     def __init__(self, n, frames=16, h=270, w=480, seed=0, with_gt=True):
-        self.n, self.frames, self.h, self.w, self.seed, self.with_gt = int(n), int(frames), int(h), int(w), int(seed), bool(with_gt)
+        self.n, self.seed, self.with_gt = int(n), int(seed), bool(with_gt)
+        per = lambda v: [int(x) for x in v] if hasattr(v, "__len__") else [int(v)] * self.n   # noqa: E731
+        self.frames, self.h, self.w = per(frames), per(h), per(w)
+        if not len(self.frames) == len(self.h) == len(self.w) == self.n:
+            raise ValueError("SyntheticSequences: one frames / h / w value per sequence")
         self._cache = {}
 
     def __len__(self):
         return self.n
+
+    def shape_of(self, sid):
+        """(T, h, W) of sequence `sid` without generating it."""
+        if not 0 <= sid < self.n:
+            raise IndexError(sid)
+        return self.frames[sid], self.h[sid], self.w[sid]
 
     def __getitem__(self, sid):
         import numpy as np
@@ -130,7 +141,7 @@ class SyntheticSequences:
             raise IndexError(sid)
         if sid in self._cache:
             return self._cache[sid]
-        T, h, w = self.frames, self.h, self.w
+        T, h, w = self.shape_of(sid)
         rng = np.random.default_rng(900000 + 7919 * self.seed + sid)
         # a slowly drifting smooth image: low-resolution noise upsampled x8, shifted by one pixel per frame
         base = rng.integers(0, 256, (h // 8 + 3, w // 8 + 3 + T)).astype(np.float32)

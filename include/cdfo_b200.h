@@ -15,6 +15,7 @@
  *   cdfo_flow_warp_fwd      arch/SIDECVSR_our.py:3068-3099  flow_warp (bilinear, zeros, align_corners=True)
  *   cdfo_mv2mvs             test_LD_37.py:83-105  mv2mvs  (+ permute at :160-161);  cdfo_mv2mvs_ra: opt/data_RA_bi.py:496-533
  *   cdfo_mv_end_fix         test_LD_37.py:209-234 modify_mv_for_end_frames
+ *   cdfo_mv_end_fix_batched the same fix-up with its own (i, max_idx) per sample (frame driver slots at different frames)
  *   cdfo_pack_c8 / unpack   layout adapters NCHW fp32 <-> channel-chunked bf16 used by the sm_100a kernels
  *   cdfo_dcn_sm100_fwd      same contraction as cdfo_dcn_fwd at the model's hot shape (C=Co=64, 3x3, s=p=d=1,
  *                           groups=1), tcgen05 implicit GEMM, bf16 operands, fp32 accumulate
@@ -86,6 +87,9 @@ int cdfo_mv2mvs(const void *mv, int mv_is_int32, float *flows, int H, int W, voi
 int cdfo_mv2mvs_ra(const void *mv_l0, const void *mv_l1, int mv_is_int32, float *flows, int H, int W, void *stream);
 /* ---- A2: in-place end-of-sequence fix-up on flows [B,7,2,H,W]; frame index i, max_idx as the caller passes. */
 int cdfo_mv_end_fix(float *flows, int B, int H, int W, int i, int max_idx, void *stream);
+/* Same fix-up, one launch for the whole batch, sample b using (i, max_idx) = i_max[2 b], i_max[2 b + 1]: i_max is a DEVICE int32
+ * table [B, 2], so a step that uses it stays capturable in a CUDA graph.  Per sample bit-identical to cdfo_mv_end_fix. */
+int cdfo_mv_end_fix_batched(float *flows, int B, int H, int W, const int *i_max, void *stream);
 
 /* ---- A9: prior embedding convs conv_expand_ufs / conv_expand_rms = nn.Conv2d(1, Co, 3, 1, 1) (arch/SIDECVSR_our.py:4383-4384,
  * :4446-4447).  x [B,1,H,W] fp32, w [Co,1,3,3], bias [Co] or NULL -> y [B,Co,H,W] fp32. */
